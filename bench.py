@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: G1 scalar-mul STARK proofs/sec (BASELINE.json `metric`), one JSON line on stdout.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--instances 1024]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--instances 1024] [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over one batch: generate_trace + prove of `--instances` G1
 scalar-muls in ONE trace (default 1024 => 2^19 rows x 781 columns = BASELINE.json configs[1], SURVEY.md
@@ -343,15 +343,24 @@ def run_ours(args, rank, world, local_rank):
     sampler.start()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record(stream)
+    last = None
     for i in range(args.steps):
         pf = step_dev(i)
         for name, ms in ctx.timings():
             stage_ms[name] = stage_ms.get(name, 0.0) + ms
-        pf.close()
+        if i + 1 < args.steps:
+            pf.close()
+        else:
+            last = pf  # read back after the timed region
     ev1.record(stream)
     barrier()
     dev_s = max_over_ranks(ev0.elapsed_time(ev1) * 1e-3)
     launches = lib.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {
+            "proof_words": u64_as_f64_halves(last.words()),
+            "results": last.results().reshape(args.instances, -1).astype(np.float64)})
+    last.close()
 
     # ---- e2e: host buffers through the C ABI ---------------------------------------------------
     barrier()
@@ -553,6 +562,28 @@ def run_ours(args, rank, world, local_rank):
         dist.destroy_process_group()
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def u64_as_f64_halves(words):
+    """uint64 words -> (n, 2) float64 [low 32 bits, high 32 bits]: a Goldilocks element does not fit float64's
+    53-bit mantissa, its two halves do, so the file holds the words exactly."""
+    import numpy as np
+    w = np.ascontiguousarray(words, dtype=np.uint64).reshape(-1)
+    return np.stack([w & np.uint64(0xFFFFFFFF), w >> np.uint64(32)], axis=1).astype(np.float64)
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each array as out_dir/<name>.npy, so that two builds can be compared output for output."""
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: outputs of {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte dump limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 _REAL_STDOUT = None
 
 
@@ -595,7 +626,15 @@ def main():
     ap.add_argument("--oversized-instances", type=int, default=8192, help="8192 G1 scalar-muls = 2^22 rows (config 5)")
     ap.add_argument("--no-full-check", action="store_true",
                     help="reference arm: skip the one full-workload proof timed before the steps")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0) as DIR/<name>.npy, float64: proof_words "
+                         "(n x 2: low and high 32 bits of each u64 proof word) and results (instances x 16-bit limbs "
+                         "of the native outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -2,11 +2,19 @@
 the bench line quotes from profiles/*_metrics.json instead of typed-in constants."""
 import json
 import os
+import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import bench  # noqa: E402
+
+
+def _words_from_halves(h):
+    return h[:, 0].astype(np.uint64) | (h[:, 1].astype(np.uint64) << np.uint64(32))
 
 
 def test_algorithmic_bytes_formulas():
@@ -39,3 +47,34 @@ def test_workload_config_names_the_baseline_workload():
     c = bench.workload_config(A)
     assert c["trace_rows"] == 1 << 19 and c["trace_columns"] == 781 and "1024 scalar-muls" in c["workload"]
     assert "model" not in c
+
+
+def test_dumped_words_are_exact_and_the_dump_is_bounded(tmp_path, monkeypatch):
+    w = np.array([0, 1, 0xFFFFFFFF, 1 << 32, 0xFFFFFFFF00000000, 0xFFFFFFFFFFFFFFFF], dtype=np.uint64)
+    h = bench.u64_as_f64_halves(w)
+    assert h.dtype == np.float64 and h.shape == (6, 2) and (_words_from_halves(h) == w).all()
+    bench.dump_outputs(str(tmp_path / "d"), {"proof_words": h})
+    assert (np.load(tmp_path / "d" / "proof_words.npy") == h).all()
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", h.nbytes - 1)
+    with pytest.raises(SystemExit):
+        bench.dump_outputs(str(tmp_path / "e"), {"proof_words": h})
+    assert not (tmp_path / "e").exists()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_is_the_last_timed_proof(gpu_ctx, tmp_path):
+    """bench.py --dump-outputs writes what its last timed step returned: step i proves batch i % 3 (seed
+    config_seed(2) + b on rank 0), so with --steps 2 that is batch 1, whose pb254_prove proof and native results
+    the dumped arrays must equal exactly."""
+    from plonky2_bn254_b200 import inputs as I
+    out = tmp_path / "dump"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1",
+                        "--instances", "3", "--no-cpu-baseline", "--no-other-configs", "--no-pipelined",
+                        "--dump-outputs", str(out)], capture_output=True, text=True, cwd=tmp_path)
+    assert r.returncode == 0, r.stderr[-3000:]
+    assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 2
+    inp, ts = I.make_inputs(I.KIND_G1, 3, I.config_seed(2) + 1)
+    pf = gpu_ctx.prove(I.KIND_G1, inp, ts)
+    words = _words_from_halves(np.load(out / "proof_words.npy"))
+    assert words.size == pf.words().size and (words == pf.words()).all()
+    assert (np.load(out / "results.npy") == pf.results().reshape(3, -1)).all()
