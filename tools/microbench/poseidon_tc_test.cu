@@ -81,7 +81,7 @@ int main(int argc, char** argv) {
     cudaEventElapsedTime(&ms_tc, e0, e1);
   }
   CK(cudaGetLastError());
-  printf("tcgen05 (ctas %d): %.3f ms, %.3f Gperm/s\n", PB_TC_CTAS, ms_tc, n * (double)reps / ms_tc * 1e-6);
+  printf("tcgen05 (ctas %d): %.3f ms, %.3f Gperm/s\n", poseidon::tc::CTAS_PER_SM, ms_tc, n * (double)reps / ms_tc * 1e-6);
   std::vector<u64> r1(12 * n), r2(12 * n);
   CK(cudaMemcpy(r1.data(), d1, 96 * n, cudaMemcpyDeviceToHost));
   CK(cudaMemcpy(r2.data(), d2, 96 * n, cudaMemcpyDeviceToHost));
