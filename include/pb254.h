@@ -141,6 +141,20 @@ int pb254_prove_sharded(pb254_ctx* ctx, int kind, const uint64_t* inputs, const 
 int pb254_generate_trace(pb254_ctx* ctx, int kind, const uint64_t* inputs, const uint64_t* timestamps,
                          size_t n_inputs, size_t min_rows, uint64_t* cols_out);
 
+/* ---- witness before proving (K13) ------------------------------------------------------------ */
+/* Chained scalar multiplications, the witness G1/G2SingleGenerator computes natively before run_once
+ * (src/generators/g1/single.rs:48-52) and g1_msm threads through `offset` (src/utils/g1_msm.rs:22-36).
+ * kind: PB254_KIND_G1 or PB254_KIND_G2. terms: n_terms rows of s, x (G1 12 words, G2 20 words), in chain order.
+ * chain_starts: n_chains + 1 indices, chain_starts[0] = 0, non-decreasing, chain_starts[n_chains] = n_terms.
+ * offsets: n_chains affine points (G1 8 words, G2 16 words). For chain c: acc = offsets[c]; for each term i of the
+ * chain, row i of inputs_out = (s_i, x_i, acc) and acc = s_i * x_i + acc; sums_out[c] = acc (may be NULL).
+ * inputs_out is in the pb254_prove wire format. At most 2^17 terms and 2^17 chains. PB254_E_INFINITY if an
+ * accumulator after the first is the point at infinity (pb254_last_error() names the lowest such chain and term);
+ * PB254_E_NOT_CANONICAL / PB254_E_NOT_ON_CURVE as pb254_prove. */
+int pb254_scalar_mul_chains(pb254_ctx* ctx, int kind, const uint64_t* terms, size_t n_terms,
+                            const uint64_t* chain_starts, size_t n_chains, const uint64_t* offsets,
+                            uint64_t* inputs_out, uint64_t* sums_out);
+
 /* ---- proving ------------------------------------------------------------------------------- */
 /* generate_trace + prove in one call, the body of run_once between
  * src/generators/g1/stark_proof.rs:154 and :163; the trace stays on the device.

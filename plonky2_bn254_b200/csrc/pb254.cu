@@ -10,6 +10,7 @@ std::atomic<unsigned long long> g_pb_launches{0};
 #include <thread>
 #include "merkle.cuh"
 #include "tracegen.h"
+#include "chains.cuh"
 #include "prover.cuh"
 #include "verify.cuh"
 
@@ -99,6 +100,61 @@ struct GatherResultsK {
     out[gid] = trace[(size_t)(reg1 + i) * n_rows + k * tg::PERIOD + (tg::PERIOD - 1)];
   }
 };
+
+template <class F>
+void scalar_mul_chains_impl(pb254_ctx* c, const u64* terms, size_t n_terms, const u64* chain_starts, size_t n_chains,
+                            const u64* offsets, u64* inputs_out, u64* sums_out) {
+  const size_t FW = tg::FieldIO<F>::WORDS, TW = 4 + 2 * FW, RW = TW + 2 * FW, n = n_terms + n_chains;
+  c->arena.reserve(chains::scratch_bytes<F>(n_terms, n_chains) +
+                   (n_terms * (TW + RW) + (n_chains + 1) + 2 * n_chains * 2 * FW) * 8 + 65536);
+  c->arena.reset();
+  c->times.clear();
+  const pbStream s = c->stream;
+  chains::Bufs<F> B;
+  u64* d_terms = c->arena.alloc_n<u64>(n_terms * TW);
+  u64* d_starts = c->arena.alloc_n<u64>(n_chains + 1);
+  u64* d_offsets = c->arena.alloc_n<u64>(n_chains * 2 * FW);
+  u64* d_rows = c->arena.alloc_n<u64>(n_terms * RW);
+  u64* d_sums = sums_out ? c->arena.alloc_n<u64>(n_chains * 2 * FW) : nullptr;
+  B.terms = d_terms;
+  B.starts = d_starts;
+  B.offsets = d_offsets;
+  B.D = c->arena.alloc_n<bn::Jac<F>>(256 * n_terms);
+  B.E = c->arena.alloc_n<bn::Jac<F>>(n);
+  B.head = c->arena.alloc_n<int>(n);
+  B.A = c->arena.alloc_n<bn::Aff<F>>(n);
+  B.err = c->arena.alloc_n<int>(1);
+  B.first_inf = c->arena.alloc_n<unsigned>(1);
+  B.n_terms = n_terms;
+  B.n_chains = n_chains;
+  if (n_terms) pb_h2d(d_terms, terms, n_terms * TW * 8, s);
+  pb_h2d(d_starts, chain_starts, (n_chains + 1) * 8, s);
+  pb_h2d(d_offsets, offsets, n_chains * 2 * FW * 8, s);
+  pb_memset(B.err, 0, sizeof(int), s);
+  pb_memset(B.first_inf, 0xff, sizeof(unsigned), s);
+  chains::run<F>(c, B, d_rows, d_sums);
+  int herr = 0;
+  unsigned first_inf = chains::NO_INF;
+  pb_d2h(&herr, B.err, sizeof(int), s);
+  pb_d2h(&first_inf, B.first_inf, sizeof(unsigned), s);
+  pb_sync(s);
+  c->times.resolve();
+  if (herr == tg::ERR_NOT_CANONICAL || herr == tg::ERR_NOT_ON_CURVE) throw_trace_error(herr);
+  if (first_inf != chains::NO_INF) {
+    // element e = i + ch + 1 holds the accumulator after term i of chain ch
+    size_t ch = 0;
+    while (ch + 1 < n_chains && chain_starts[ch + 1] + ch + 1 <= first_inf) ch++;
+    const size_t i = first_inf - ch - 1;
+    throw Pb254Error(PB254_E_INFINITY, "chain " + std::to_string(ch) + ", term " + std::to_string(i) + " (index " +
+                                           std::to_string(i - chain_starts[ch]) +
+                                           " in the chain): the accumulator s*x + offset is the point at infinity, "
+                                           "unsupported by design");
+  }
+  throw_trace_error(herr);
+  if (n_terms) pb_d2h(inputs_out, d_rows, n_terms * RW * 8, s);
+  if (sums_out) pb_d2h(sums_out, d_sums, n_chains * 2 * FW * 8, s);
+  pb_sync(s);
+}
 
 struct PermuteK {
   const u64* in;
@@ -279,6 +335,28 @@ int pb254_generate_trace(pb254_ctx* c, int kind, const uint64_t* inputs, const u
     pb_sync(c->stream);
     c->times.resolve();
     throw_trace_error(herr);
+  });
+}
+
+int pb254_scalar_mul_chains(pb254_ctx* c, int kind, const uint64_t* terms, size_t n_terms,
+                            const uint64_t* chain_starts, size_t n_chains, const uint64_t* offsets,
+                            uint64_t* inputs_out, uint64_t* sums_out) {
+  return guarded([&] {
+    need_ctx(c);
+    need(kind == PB254_KIND_G1 || kind == PB254_KIND_G2, "kind must be PB254_KIND_G1 or PB254_KIND_G2");
+    need(chain_starts != nullptr, "null chain_starts");
+    need(n_terms <= chains::MAX_TERMS && n_chains <= chains::MAX_CHAINS, "more than 2^17 terms or chains");
+    need(n_terms == 0 || (terms && inputs_out), "null terms or inputs_out");
+    need(n_chains == 0 || offsets, "null offsets");
+    need(chain_starts[0] == 0 && chain_starts[n_chains] == n_terms,
+         "chain_starts must begin at 0 and end at n_terms");
+    for (size_t k = 0; k < n_chains; k++) need(chain_starts[k] <= chain_starts[k + 1], "chain_starts must not decrease");
+    if (n_chains == 0) return;
+    PbDeviceGuard device_guard(c->device);
+    if (kind == PB254_KIND_G1)
+      scalar_mul_chains_impl<bn::F1>(c, terms, n_terms, chain_starts, n_chains, offsets, inputs_out, sums_out);
+    else
+      scalar_mul_chains_impl<bn::F2>(c, terms, n_terms, chain_starts, n_chains, offsets, inputs_out, sums_out);
   });
 }
 

@@ -328,6 +328,28 @@ class Context:
                                                      C.c_size_t(min_rows), _p(cols)))
         return cols
 
+    # ---- witness before proving -------------------------------------------------------------
+    def scalar_mul_chains(self, kind, terms, chain_starts, offsets):
+        """pb254_scalar_mul_chains: chain c starts at offsets[c] and each of its terms (s, x) adds s * x.
+        terms (n_terms, 12 | 20) rows of s, x in chain order; chain_starts (n_chains + 1,) with chain_starts[0] = 0 and
+        chain_starts[-1] = n_terms; offsets (n_chains, 8 | 16) affine points. Returns (inputs, sums): inputs
+        (n_terms, input_words(kind)) pb254_prove rows (s, x, accumulator before the term), sums (n_chains, 8 | 16) the
+        final accumulators."""
+        fw = 4 if kind == KIND_G1 else 8             # any other kind is rejected by the library
+        terms = _u64(terms)
+        starts = _u64(chain_starts).reshape(-1)
+        offsets = _u64(offsets)
+        n_chains = starts.size - 1
+        if kind in (KIND_G1, KIND_G2) and (terms.ndim != 2 or terms.shape[1] != 4 + 2 * fw or n_chains < 0 or
+                                           offsets.size != n_chains * 2 * fw):
+            raise Pb254Error(6, f"terms must be (n, {4 + 2 * fw}) and offsets (len(chain_starts) - 1, {2 * fw})")
+        inputs = np.empty((terms.shape[0], 4 + 4 * fw), dtype=np.uint64)
+        sums = np.empty((n_chains, 2 * fw), dtype=np.uint64)
+        self.L.check(self.L.lib.pb254_scalar_mul_chains(self._h, C.c_int(kind), _p(terms), C.c_size_t(terms.shape[0]),
+                                                        _p(starts), C.c_size_t(n_chains), _p(offsets), _p(inputs),
+                                                        _p(sums)))
+        return inputs, sums
+
     # ---- proving --------------------------------------------------------------------------
     def prove(self, kind, inputs, timestamps, min_rows=1 << 16, config: Config | None = None, keep_debug=False):
         """generate_trace + prove on the device; returns a :class:`Proof`."""

@@ -10,6 +10,8 @@ reference that produce large batches of hot-path work items.
   with a random offset (:195-208) followed by ``- offset``. A batch of messages is a batch of
   ``G2ScalarMulInput {s: cofactor, x: mapped point, offset}``; ``hash_to_g2_outputs`` removes the offsets from the
   STARK's native results.
+* ``g1_msm`` (src/utils/g1_msm.rs:22-36): a chain of G1 scalar-muls threaded through ``offset`` from a random subgroup
+  point; ``g1_msm_inputs`` builds the batch on the device (``Context.scalar_mul_chains``) and returns the MSM.
 
 Host-side, pure Python / numpy: this is workload generation (what the reference's witness generators do on the CPU
 before they reach ``run_once``), not part of the prover. The Poseidon permutation is injected (``Context.poseidon_permute``
@@ -227,3 +229,53 @@ def hash_to_g2_outputs(results, offsets):
     per instance)."""
     res = np.asarray(results).reshape(-1, 64)
     return [g2_add(_g2_from_limbs16(r), g2_neg(off)) for r, off in zip(res, offsets)]
+
+
+# ---- g1_msm (src/utils/g1_msm.rs:22-36) ----------------------------------------------------------------------------
+def g1_neg(P):
+    return None if P is None else (P[0], -P[1] % BN254_P)
+
+
+def g1_add(P, Q):
+    """Affine addition on G1; None is the point at infinity."""
+    if P is None:
+        return Q
+    if Q is None:
+        return P
+    if P[0] == Q[0]:
+        if (P[1] + Q[1]) % BN254_P == 0:
+            return None
+        lam = 3 * P[0] * P[0] * pow(2 * P[1], -1, BN254_P) % BN254_P
+    else:
+        lam = (Q[1] - P[1]) * pow(Q[0] - P[0], -1, BN254_P) % BN254_P
+    x = (lam * lam - P[0] - Q[0]) % BN254_P
+    return (x, (lam * (P[0] - x) - P[1]) % BN254_P)
+
+
+def g1_mul(k: int, P):
+    acc = None
+    for bit in bin(k)[2:]:
+        acc = g1_add(acc, acc)
+        if bit == "1":
+            acc = g1_add(acc, P)
+    return acc
+
+
+def g1_msm_inputs(ctx, scalars, points, seed: int):
+    """The G1ScalarMulInput batch of ``g1_msm(scalars, points)``, built on the device: one chain that starts at a random
+    subgroup point acc_0 (drawn from ``SplitMix64(seed)`` as ``hash_to_g2_inputs`` draws its offsets) and adds
+    s_i * x_i term by term, so that row i is (s_i, x_i, acc_i) (``Context.scalar_mul_chains``).
+    scalars: ints < 2^256; points: affine G1 points (x, y). Returns (inputs[n, 20], timestamps[n], msm) with
+    msm = acc_n - acc_0 as an affine point, None for the point at infinity."""
+    rng = I.SplitMix64(seed)
+    k = 0
+    while k % BN254_R == 0:
+        k = rng.bits256() & ((1 << 254) - 1)
+    off = I.scalar_mul_gen(I.KIND_G1, k)
+    terms = np.array([I._words(int(s)) + I._words(p[0]) + I._words(p[1]) for s, p in zip(scalars, points)],
+                     dtype=np.uint64).reshape(-1, 12)
+    starts = np.array([0, terms.shape[0]], dtype=np.uint64)
+    inputs, sums = ctx.scalar_mul_chains(I.KIND_G1, terms, starts, np.array(I._words(off[0]) + I._words(off[1]),
+                                                                           dtype=np.uint64))
+    total = (_int256(sums[0, :4]), _int256(sums[0, 4:]))
+    return inputs, np.arange(inputs.shape[0], dtype=np.uint64), g1_add(total, g1_neg(off))

@@ -165,6 +165,54 @@ impl Context {
         Ok(Proved { proof: decode_proof(&blob)?, blob, results })
     }
 
+    /// `pb254_scalar_mul_chains`: the witness `G1SingleGenerator` / `G2SingleGenerator` compute before run_once
+    /// (src/generators/g1/single.rs:48-52). `terms` holds n rows of s, x (G1 12 words, G2 20 words) in chain order,
+    /// `chain_starts` n_chains + 1 indices (first 0, last n, non-decreasing), `offsets` one affine point per chain
+    /// (G1 8 words, G2 16 words). Returns (inputs, sums): the `pack_*` wire rows (s, x, accumulator before the term),
+    /// ready for `prove`, and the final accumulator of every chain.
+    pub fn scalar_mul_chains(&self, kind: i32, terms: &[u64], chain_starts: &[u64], offsets: &[u64]) -> Result<(Vec<u64>, Vec<u64>)> {
+        let fw = match kind {
+            sys::PB254_KIND_G1 => 4,
+            sys::PB254_KIND_G2 => 8,
+            _ => return Err(anyhow!("scalar_mul_chains: kind must be PB254_KIND_G1 or PB254_KIND_G2")),
+        };
+        let n_chains = chain_starts.len().checked_sub(1).ok_or_else(|| anyhow!("empty chain_starts"))?;
+        if terms.len() % (4 + 2 * fw) != 0 || offsets.len() != n_chains * 2 * fw {
+            return Err(anyhow!("scalar_mul_chains: terms / offsets do not match the kind and chain_starts"));
+        }
+        let n_terms = terms.len() / (4 + 2 * fw);
+        let mut inputs = vec![0u64; n_terms * (4 + 4 * fw)];
+        let mut sums = vec![0u64; n_chains * 2 * fw];
+        check(unsafe {
+            sys::pb254_scalar_mul_chains(self.0, kind, terms.as_ptr(), n_terms, chain_starts.as_ptr(), n_chains,
+                                         offsets.as_ptr(), inputs.as_mut_ptr(), sums.as_mut_ptr())
+        })?;
+        Ok((inputs, sums))
+    }
+
+    /// The G1ScalarMulInput batch of `g1_msm(scalars, points)` (src/utils/g1_msm.rs:22-36) as one chain from a
+    /// random subgroup point `offset`: returns (the `pack_g1` words of the batch, sum s_i x_i), the MSM being
+    /// acc_N - acc_0. An accumulator at infinity is an error, as in the reference (g1_msm.rs:20-21).
+    pub fn g1_msm(&self, scalars: &[BigUint], points: &[G1Affine], offset: &G1Affine) -> Result<(Vec<u64>, G1Affine)> {
+        use ark_ec::{AffineRepr, CurveGroup};
+        if scalars.len() != points.len() {
+            return Err(anyhow!("g1_msm: {} scalars for {} points", scalars.len(), points.len()));
+        }
+        let mut terms = Vec::with_capacity(points.len() * 12);
+        for (s, x) in scalars.iter().zip(points) {
+            push_biguint(&mut terms, s);
+            push_fq(&mut terms, &x.x);
+            push_fq(&mut terms, &x.y);
+        }
+        let mut off = Vec::with_capacity(8);
+        push_fq(&mut off, &offset.x);
+        push_fq(&mut off, &offset.y);
+        let (inputs, sums) = self.scalar_mul_chains(sys::PB254_KIND_G1, &terms, &[0, points.len() as u64], &off)?;
+        let fq = |w: &[u64]| Fq::from_bigint(BigInt([w[0], w[1], w[2], w[3]])).expect("canonical");
+        let acc = G1Affine::new_unchecked(fq(&sums[..4]), fq(&sums[4..]));
+        Ok((inputs, (acc.into_group() - offset.into_group()).into_affine()))
+    }
+
     /// `generate_trace(&inputs, min_rows)` + `prove` (run_once lines 154-163) for `kind`; `words` as produced by
     /// `pack_*`; `config` None = `StarkConfig::standard_fast_config()`.
     pub fn prove(&self, kind: i32, words: &[u64], timestamps: &[u64], min_rows: usize, config: Option<&StarkConfig>) -> Result<Proved> {
