@@ -155,6 +155,24 @@ int pb254_scalar_mul_chains(pb254_ctx* ctx, int kind, const uint64_t* terms, siz
                             const uint64_t* chain_starts, size_t n_chains, const uint64_t* offsets,
                             uint64_t* inputs_out, uint64_t* sums_out);
 
+/* The Shallue-van de Woestijne map of HashToG2::map_to_g2 (src/utils/hash_to_g2.rs:113-147), before cofactor
+ * clearing. us: n values u in Fq2, 8 words each (c0, c1). points_out: n affine points of the G2 curve, 16 words each
+ * (x.c0, x.c1, y.c0, y.c1). Square roots as ark-ff computes them: a^((p+1)/4) in Fq, the complex method in Fq2; the
+ * sign of y follows sgn(u) (src/fields/sgn.rs:20-27). At most 2^17 values. PB254_E_NOT_CANONICAL for a coordinate
+ * >= p, PB254_E_BAD_ARG for an exceptional u (tv1 * tv2 = 0); pb254_last_error() names the lowest such index. */
+int pb254_map_to_g2(pb254_ctx* ctx, const uint64_t* us, size_t n, uint64_t* points_out);
+
+/* HashToG2::hash_to_g2 (src/utils/hash_to_g2.rs:76-148) of n messages of msg_len canonical Goldilocks elements each
+ * (row-major; msg_len = 0 is valid), with the cofactor clearing of the circuit (:195-208) as pb254_prove G2 rows.
+ * u_i = hash_to_fq2(m_i) (the plonky2 Challenger, :76-87), x_i = map_to_g2(u_i), k_i = the 254 low bits of the
+ * SplitMix64(seed) draws 4i+1 .. 4i+4 (little endian), offset_i = k_i * G2.
+ * inputs_out: n rows of 36 words (s = the G2 cofactor, x_i, offset_i). hashes_out: n affine points of 16 words,
+ * cofactor * x_i, the hash_to_g2 output. At most 2^17 messages and 2^24 message elements in all. Errors name the
+ * lowest failing message: PB254_E_NOT_CANONICAL (an element >= 2^64 - 2^32 + 1), PB254_E_BAD_ARG (an exceptional u,
+ * or k_i = 0 mod r), PB254_E_INFINITY (cofactor * x_i + offset_i or cofactor * x_i at infinity). */
+int pb254_hash_to_g2(pb254_ctx* ctx, const uint64_t* messages, size_t n, size_t msg_len, uint64_t seed,
+                     uint64_t* inputs_out, uint64_t* hashes_out);
+
 /* ---- proving ------------------------------------------------------------------------------- */
 /* generate_trace + prove in one call, the body of run_once between
  * src/generators/g1/stark_proof.rs:154 and :163; the trace stays on the device.

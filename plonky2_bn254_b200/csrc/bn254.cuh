@@ -168,8 +168,20 @@ PB_HD Fq inv(const Fq& a) {
   }
   return r;
 }
-
-// canonical integer <-> 4 little-endian u64 words / 16 x 16-bit limbs
+// a^e for an exponent given as 8 little-endian 32-bit limbs, square-and-multiply from bit 255. The limb of each step
+// is picked by unrolled selects, so that a constant exponent stays in registers (no local-memory indexing).
+PB_HD Fq pow(const Fq& a, const u32 (&e)[8]) {
+  Fq r = one();
+#pragma unroll 1
+  for (int i = 255; i >= 0; i--) {
+    r = sqr(r);
+    u32 w = e[0];
+#pragma unroll
+    for (int k = 1; k < 8; k++) w = (i >> 5) == k ? e[k] : w;
+    if ((w >> (i & 31)) & 1) r = mul(r, a);
+  }
+  return r;
+}
 PB_HD Fq from_words(const u64 w[4]) {
   Fq r;
 #pragma unroll

@@ -126,15 +126,7 @@ template <class F>
 struct FindInfK {
   Bufs<F> B;
   PB_HD void operator()(size_t e) const {
-    if (!F::is_zero(B.E[e].Z)) return;
-#ifdef __CUDA_ARCH__
-    atomicMin(B.first_inf, (unsigned)e);
-#else
-    unsigned cur = __atomic_load_n(B.first_inf, __ATOMIC_RELAXED);
-    while ((unsigned)e < cur &&
-           !__atomic_compare_exchange_n(B.first_inf, &cur, (unsigned)e, false, __ATOMIC_RELAXED, __ATOMIC_RELAXED)) {
-    }
-#endif
+    if (F::is_zero(B.E[e].Z)) tg::set_lowest(B.first_inf, (unsigned)e);
   }
 };
 
@@ -191,44 +183,53 @@ struct ScanK {  // one chain, serially
 };
 template <class F>
 struct AffK {
-  Bufs<F> B;
+  const bn::Jac<F>* src;
+  bn::Aff<F>* dst;
+  int* err;
   PB_HD void operator()(size_t e) const {
-    const bn::Jac<F> p = B.E[e];
+    const bn::Jac<F> p = src[e];
     if (F::is_zero(p.Z)) {
-      tg::set_err(B.err, tg::ERR_INFINITY);
-      B.A[e].x = B.A[e].y = F::zero();
+      tg::set_err(err, tg::ERR_INFINITY);
+      dst[e].x = dst[e].y = F::zero();
       return;
     }
     const typename F::T zi = F::inv(p.Z), zi2 = F::sqr(zi);
-    B.A[e].x = F::mul(p.X, zi2);
-    B.A[e].y = F::mul(p.Y, F::mul(zi, zi2));
+    dst[e].x = F::mul(p.X, zi2);
+    dst[e].y = F::mul(p.Y, F::mul(zi, zi2));
   }
 };
 #else
 // ---- device-only block code -------------------------------------------------------------------------------------
-// 1b. one warp per term: lane l adds D_(8l .. 8l+7) of the set bits, then a 5-level tree adds the lanes. The partial
-// sums live in shared memory, so that an addition's operands are loaded as it needs them (F2: no spills at 255 regs).
-static constexpr int SUM_WARPS = 4;
+// The sum over the set bits of a 256-bit scalar w of the table points D[j * stride], one warp per scalar: lane l adds
+// the entries of bits 8l .. 8l+7, then a 5-level tree adds the lanes; the sum is left in p[0]. The partial sums live
+// in shared memory (p: 32 entries of this warp), so that an addition's operands are loaded as it needs them (F2: no
+// spills at 255 registers).
 template <class F>
-__global__ void __launch_bounds__(32 * SUM_WARPS) k_chain_sum(Bufs<F> B) {
-  __shared__ bn::Jac<F> part[SUM_WARPS][32];
-  const size_t i = (size_t)blockIdx.x * SUM_WARPS + (threadIdx.x >> 5);
-  if (i >= B.n_terms) return;  // whole warps
+__device__ __forceinline__ void warp_bit_sum(bn::Jac<F>* p, const u64* w, const bn::Jac<F>* D, size_t stride) {
   const int lane = threadIdx.x & 31;
-  bn::Jac<F>* p = part[threadIdx.x >> 5];
-  const u64* w = B.terms + i * (4 + 2 * FieldIO<F>::WORDS);
   const u32 bits = (u32)(w[lane >> 3] >> ((lane & 7) * 8)) & 0xffu;
   p[lane] = infinity<F>();
 #pragma unroll 1
   for (int t = 0; t < 8; t++)
-    if ((bits >> t) & 1) p[lane] = bn::jac_add_complete<F>(p[lane], B.D[(size_t)(8 * lane + t) * B.n_terms + i]);
+    if ((bits >> t) & 1) p[lane] = bn::jac_add_complete<F>(p[lane], D[(size_t)(8 * lane + t) * stride]);
   __syncwarp();
 #pragma unroll 1
   for (int d = 16; d >= 1; d >>= 1) {
     if (lane < d) p[lane] = bn::jac_add_complete<F>(p[lane], p[lane + d]);
     __syncwarp();
   }
-  if (lane == 0) {
+}
+
+// 1b. one warp per term: s_i x_i from the doublings D_j = 2^j x_i of the set bits of s_i
+static constexpr int SUM_WARPS = 4;
+template <class F>
+__global__ void __launch_bounds__(32 * SUM_WARPS) k_chain_sum(Bufs<F> B) {
+  __shared__ bn::Jac<F> part[SUM_WARPS][32];
+  const size_t i = (size_t)blockIdx.x * SUM_WARPS + (threadIdx.x >> 5);
+  if (i >= B.n_terms) return;  // whole warps
+  bn::Jac<F>* p = part[threadIdx.x >> 5];
+  warp_bit_sum<F>(p, B.terms + i * (4 + 2 * FieldIO<F>::WORDS), B.D + i, B.n_terms);
+  if ((threadIdx.x & 31) == 0) {
     const size_t e = i + chain_of_term(B.starts, B.n_chains, i) + 1;
     B.E[e] = p[0];
     B.head[e] = 0;
@@ -293,6 +294,20 @@ void seg_scan(Arena& ar, bn::Jac<F>* v, int* head, size_t n, pbStream s) {
 }
 #endif
 
+// dst[e] = affine(src[e]), e < n; a point at infinity flags tg::ERR_INFINITY
+template <class F>
+void to_affine(const bn::Jac<F>* src, bn::Aff<F>* dst, size_t n, int* err, pbStream s) {
+#if PB_HOSTSIM
+  pb_launch("to affine", AffK<F>{src, dst, err}, n, s);
+#else
+  const size_t threads = (n + tg::AFF_CH - 1) / tg::AFF_CH;
+  if (!threads) return;
+  tg::k_to_affine<F><<<(unsigned)((threads + 127) / 128), 128, 0, s>>>(src, dst, n, 0, err);
+  g_pb_launches++;
+  pb_check_last("to affine");
+#endif
+}
+
 // scratch bytes for n_terms / n_chains (the scan's aggregate levels included)
 template <class F>
 size_t scratch_bytes(size_t n_terms, size_t n_chains) {
@@ -327,14 +342,7 @@ void run(pb254_ctx* c, Bufs<F> B, u64* d_rows, u64* d_sums) {
   pb_launch("chains infinity", FindInfK<F>{B}, n, s, 128);
   c->times.end(t1, s);
   int t2 = c->times.begin("chains affine", s);
-#if PB_HOSTSIM
-  pb_launch("chains affine", AffK<F>{B}, n, s);
-#else
-  const size_t aff_threads = (n + tg::AFF_CH - 1) / tg::AFF_CH;
-  tg::k_to_affine<F><<<(unsigned)((aff_threads + 127) / 128), 128, 0, s>>>(B.E, B.A, n, 0, B.err);
-  g_pb_launches++;
-  pb_check_last("chains affine");
-#endif
+  to_affine<F>(B.E, B.A, n, B.err, s);
   pb_launch("chains rows", RowsK<F>{B, d_rows}, B.n_terms, s, 128);
   if (d_sums) pb_launch("chains sums out", SumsK<F>{B, d_sums}, B.n_chains, s, 128);
   c->times.end(t2, s);

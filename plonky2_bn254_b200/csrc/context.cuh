@@ -118,4 +118,5 @@ struct pb254_ctx {
   ntt::TableSet tables;
   Arena arena;
   StageTimes times;
+  void* g2_pow2 = nullptr;  // hash_to_g2's fixed-base table 2^j G2 (h2g2::TableK), built by the first call
 };

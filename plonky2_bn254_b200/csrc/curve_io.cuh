@@ -16,6 +16,16 @@ PB_HD void set_err(int* err, int code) {
   }
 #endif
 }
+// *slot = min(*slot, v): the lowest failing index of a batch (slots start at 0xffffffff)
+PB_HD void set_lowest(unsigned* slot, unsigned v) {
+#ifdef __CUDA_ARCH__
+  atomicMin(slot, v);
+#else
+  unsigned cur = __atomic_load_n(slot, __ATOMIC_RELAXED);
+  while (v < cur && !__atomic_compare_exchange_n(slot, &cur, v, false, __ATOMIC_RELAXED, __ATOMIC_RELAXED)) {
+  }
+#endif
+}
 
 PB_HD bool words_lt_p(const u64* w4) {
   bn::Fq t = bn::from_words(w4);

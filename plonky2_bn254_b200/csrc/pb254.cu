@@ -11,6 +11,7 @@ std::atomic<unsigned long long> g_pb_launches{0};
 #include "merkle.cuh"
 #include "tracegen.h"
 #include "chains.cuh"
+#include "hash_to_g2.cuh"
 #include "prover.cuh"
 #include "verify.cuh"
 
@@ -101,21 +102,15 @@ struct GatherResultsK {
   }
 };
 
+// The chains of pb254_scalar_mul_chains on device buffers (terms, starts and offsets uploaded, d_rows and d_sums
+// allocated; d_sums may be null), with scratch from the arena. Decodes the errors (the host chain_starts name the
+// failing chain and term) and copies the rows and sums to whichever of inputs_out / sums_out is non-null.
 template <class F>
-void scalar_mul_chains_impl(pb254_ctx* c, const u64* terms, size_t n_terms, const u64* chain_starts, size_t n_chains,
-                            const u64* offsets, u64* inputs_out, u64* sums_out) {
-  const size_t FW = tg::FieldIO<F>::WORDS, TW = 4 + 2 * FW, RW = TW + 2 * FW, n = n_terms + n_chains;
-  c->arena.reserve(chains::scratch_bytes<F>(n_terms, n_chains) +
-                   (n_terms * (TW + RW) + (n_chains + 1) + 2 * n_chains * 2 * FW) * 8 + 65536);
-  c->arena.reset();
-  c->times.clear();
+void run_chains(pb254_ctx* c, const u64* d_terms, const u64* d_starts, const u64* d_offsets, size_t n_terms,
+                const u64* chain_starts, size_t n_chains, u64* d_rows, u64* d_sums, u64* inputs_out, u64* sums_out) {
+  const size_t FW = tg::FieldIO<F>::WORDS, RW = 4 + 4 * FW, n = n_terms + n_chains;
   const pbStream s = c->stream;
   chains::Bufs<F> B;
-  u64* d_terms = c->arena.alloc_n<u64>(n_terms * TW);
-  u64* d_starts = c->arena.alloc_n<u64>(n_chains + 1);
-  u64* d_offsets = c->arena.alloc_n<u64>(n_chains * 2 * FW);
-  u64* d_rows = c->arena.alloc_n<u64>(n_terms * RW);
-  u64* d_sums = sums_out ? c->arena.alloc_n<u64>(n_chains * 2 * FW) : nullptr;
   B.terms = d_terms;
   B.starts = d_starts;
   B.offsets = d_offsets;
@@ -127,9 +122,6 @@ void scalar_mul_chains_impl(pb254_ctx* c, const u64* terms, size_t n_terms, cons
   B.first_inf = c->arena.alloc_n<unsigned>(1);
   B.n_terms = n_terms;
   B.n_chains = n_chains;
-  if (n_terms) pb_h2d(d_terms, terms, n_terms * TW * 8, s);
-  pb_h2d(d_starts, chain_starts, (n_chains + 1) * 8, s);
-  pb_h2d(d_offsets, offsets, n_chains * 2 * FW * 8, s);
   pb_memset(B.err, 0, sizeof(int), s);
   pb_memset(B.first_inf, 0xff, sizeof(unsigned), s);
   chains::run<F>(c, B, d_rows, d_sums);
@@ -151,8 +143,137 @@ void scalar_mul_chains_impl(pb254_ctx* c, const u64* terms, size_t n_terms, cons
                                            "unsupported by design");
   }
   throw_trace_error(herr);
-  if (n_terms) pb_d2h(inputs_out, d_rows, n_terms * RW * 8, s);
+  if (n_terms && inputs_out) pb_d2h(inputs_out, d_rows, n_terms * RW * 8, s);
   if (sums_out) pb_d2h(sums_out, d_sums, n_chains * 2 * FW * 8, s);
+  pb_sync(s);
+}
+
+template <class F>
+void scalar_mul_chains_impl(pb254_ctx* c, const u64* terms, size_t n_terms, const u64* chain_starts, size_t n_chains,
+                            const u64* offsets, u64* inputs_out, u64* sums_out) {
+  const size_t FW = tg::FieldIO<F>::WORDS, TW = 4 + 2 * FW, RW = TW + 2 * FW;
+  c->arena.reserve(chains::scratch_bytes<F>(n_terms, n_chains) +
+                   (n_terms * (TW + RW) + (n_chains + 1) + 2 * n_chains * 2 * FW) * 8 + 65536);
+  c->arena.reset();
+  c->times.clear();
+  const pbStream s = c->stream;
+  u64* d_terms = c->arena.alloc_n<u64>(n_terms * TW);
+  u64* d_starts = c->arena.alloc_n<u64>(n_chains + 1);
+  u64* d_offsets = c->arena.alloc_n<u64>(n_chains * 2 * FW);
+  u64* d_rows = c->arena.alloc_n<u64>(n_terms * RW);
+  u64* d_sums = sums_out ? c->arena.alloc_n<u64>(n_chains * 2 * FW) : nullptr;
+  if (n_terms) pb_h2d(d_terms, terms, n_terms * TW * 8, s);
+  pb_h2d(d_starts, chain_starts, (n_chains + 1) * 8, s);
+  pb_h2d(d_offsets, offsets, n_chains * 2 * FW * 8, s);
+  run_chains<F>(c, d_terms, d_starts, d_offsets, n_terms, chain_starts, n_chains, d_rows, d_sums, inputs_out, sums_out);
+}
+
+// the lowest failing message (or u) of each h2g2::BAD_* slot, checked in stage order
+void throw_h2g2_error(const unsigned bad[h2g2::N_BAD]) {
+  static const struct {
+    int code;
+    const char* what;
+  } kinds[h2g2::N_BAD] = {
+      {PB254_E_NOT_CANONICAL, "a message element >= the Goldilocks prime or a u coordinate >= p"},
+      {PB254_E_BAD_ARG, "exceptional u of the SvdW map (tv1 * tv2 = 0)"},
+      {PB254_E_BAD_ARG, "the offset scalar k is 0 mod r"},
+      {PB254_E_INFINITY, "cofactor * x is the point at infinity"},
+  };
+  for (int k = 0; k < h2g2::N_BAD; k++)
+    if (bad[k] != chains::NO_INF)
+      throw Pb254Error(kinds[k].code, "index " + std::to_string(bad[k]) + ": " + kinds[k].what);
+}
+void check_h2g2(pb254_ctx* c, const unsigned* d_bad) {
+  unsigned bad[h2g2::N_BAD];
+  pb_d2h(bad, d_bad, sizeof(bad), c->stream);
+  pb_sync(c->stream);
+  throw_h2g2_error(bad);
+}
+
+void map_to_g2_impl(pb254_ctx* c, const u64* us, size_t n, u64* points_out) {
+  c->arena.reserve(n * (8 * 8 + sizeof(h2g2::Fq2) + sizeof(h2g2::Aff) + 16 * 8) + 65536);
+  c->arena.reset();
+  c->times.clear();
+  const pbStream s = c->stream;
+  u64* d_us = c->arena.alloc_n<u64>(n * 8);
+  h2g2::Fq2* d_u = c->arena.alloc_n<h2g2::Fq2>(n);
+  h2g2::Aff* d_pts = c->arena.alloc_n<h2g2::Aff>(n);
+  u64* d_out = c->arena.alloc_n<u64>(n * 16);
+  unsigned* d_bad = c->arena.alloc_n<unsigned>(h2g2::N_BAD);
+  pb_h2d(d_us, us, n * 64, s);
+  pb_memset(d_bad, 0xff, h2g2::N_BAD * sizeof(unsigned), s);
+  const int t0 = c->times.begin("h2g2 map", s);
+  pb_launch("h2g2 load u", h2g2::LoadUK{d_us, d_u, d_bad}, n, s, 128);
+  pb_launch("h2g2 map", h2g2::MapK{d_u, d_pts, d_bad}, n, s, 128);
+  pb_launch("h2g2 points", h2g2::PutK{d_pts, d_out, 16}, n, s, 128);
+  c->times.end(t0, s);
+  check_h2g2(c, d_bad);
+  c->times.resolve();
+  pb_d2h(points_out, d_out, n * 128, s);
+  pb_sync(s);
+}
+
+void hash_to_g2_impl(pb254_ctx* c, const u64* messages, size_t n, size_t msg_len, u64 seed, u64* inputs_out,
+                     u64* hashes_out) {
+  using namespace h2g2;
+  typedef bn::F2 F;
+  const size_t TW = 20, RW = 36, PW = 16;
+  c->arena.reserve(chains::scratch_bytes<F>(n, n) + n * msg_len * 8 +
+                   n * (sizeof(Fq2) + 2 * sizeof(Aff) + 2 * sizeof(Jac) + (TW + 4 + PW + 1 + RW + 2 * PW) * 8) +
+                   65536);
+  c->arena.reset();
+  c->times.clear();
+  const pbStream s = c->stream;
+  if (!c->g2_pow2) {
+    c->g2_pow2 = pb_dev_alloc(TABLE_POINTS * sizeof(Jac));
+    pb_launch("h2g2 table", TableK{(Jac*)c->g2_pow2}, 1, s, 32);
+  }
+  u64* d_msgs = c->arena.alloc_n<u64>(n * msg_len + 1);
+  Fq2* d_u = c->arena.alloc_n<Fq2>(n);
+  Aff* d_pts = c->arena.alloc_n<Aff>(n);
+  u64* d_terms = c->arena.alloc_n<u64>(n * TW);
+  u64* d_k = c->arena.alloc_n<u64>(n * 4);
+  Jac* d_jac = c->arena.alloc_n<Jac>(n);
+  u64* d_offsets = c->arena.alloc_n<u64>(n * PW);
+  u64* d_starts = c->arena.alloc_n<u64>(n + 1);
+  u64* d_rows = c->arena.alloc_n<u64>(n * RW);
+  u64* d_sums = c->arena.alloc_n<u64>(n * PW);
+  u64* d_hashes = c->arena.alloc_n<u64>(n * PW);
+  unsigned* d_bad = c->arena.alloc_n<unsigned>(N_BAD);
+  int* d_err = c->arena.alloc_n<int>(1);  // the affine passes' flag: their points are never at infinity (d_bad)
+  std::vector<u64> starts(n + 1);
+  for (size_t i = 0; i <= n; i++) starts[i] = i;
+  if (msg_len) pb_h2d(d_msgs, messages, n * msg_len * 8, s);
+  pb_h2d(d_starts, starts.data(), (n + 1) * 8, s);
+  pb_memset(d_bad, 0xff, N_BAD * sizeof(unsigned), s);
+  pb_memset(d_err, 0, sizeof(int), s);
+
+  int t = c->times.begin("h2g2 hash", s);
+  pb_launch("h2g2 hash", HashK{d_msgs, msg_len, d_u, d_bad}, n, s, 128);
+  c->times.end(t, s);
+  t = c->times.begin("h2g2 map", s);
+  pb_launch("h2g2 map", MapK{d_u, d_pts, d_bad}, n, s, 128);
+  pb_launch("h2g2 terms", CofactorK{d_terms}, n, s, 128);
+  pb_launch("h2g2 points", PutK{d_pts, d_terms + 4, TW}, n, s, 128);
+  c->times.end(t, s);
+  t = c->times.begin("h2g2 offsets", s);
+  pb_launch("h2g2 draw", DrawK{seed, d_k, d_bad}, n, s, 128);
+  fixed_base((const Jac*)c->g2_pow2, d_k, n, d_jac, s);
+  chains::to_affine<F>(d_jac, d_pts, n, d_err, s);
+  pb_launch("h2g2 offsets out", PutK{d_pts, d_offsets, PW}, n, s, 128);
+  c->times.end(t, s);
+  check_h2g2(c, d_bad);
+
+  run_chains<F>(c, d_terms, d_starts, d_offsets, n, starts.data(), n, d_rows, d_sums, inputs_out, nullptr);
+
+  t = c->times.begin("h2g2 outputs", s);
+  pb_launch("h2g2 sub offset", SubOffsetK{d_sums, d_offsets, d_jac, d_bad}, n, s, 128);
+  chains::to_affine<F>(d_jac, d_pts, n, d_err, s);
+  pb_launch("h2g2 hashes out", PutK{d_pts, d_hashes, PW}, n, s, 128);
+  c->times.end(t, s);
+  check_h2g2(c, d_bad);
+  c->times.resolve();
+  pb_d2h(hashes_out, d_hashes, n * PW * 8, s);
   pb_sync(s);
 }
 
@@ -209,6 +330,7 @@ void pb254_ctx_destroy(pb254_ctx* c) {
   c->times.clear();
   c->tables.destroy();
   c->arena.destroy();
+  if (c->g2_pow2) pb_dev_free(c->g2_pow2);
 #if !PB_HOSTSIM
   if (c->own_stream) cudaStreamDestroy(c->stream);
 #endif
@@ -357,6 +479,30 @@ int pb254_scalar_mul_chains(pb254_ctx* c, int kind, const uint64_t* terms, size_
       scalar_mul_chains_impl<bn::F1>(c, terms, n_terms, chain_starts, n_chains, offsets, inputs_out, sums_out);
     else
       scalar_mul_chains_impl<bn::F2>(c, terms, n_terms, chain_starts, n_chains, offsets, inputs_out, sums_out);
+  });
+}
+
+int pb254_map_to_g2(pb254_ctx* c, const uint64_t* us, size_t n, uint64_t* points_out) {
+  return guarded([&] {
+    need_ctx(c);
+    need(n <= h2g2::MAX_N, "more than 2^17 values");
+    if (n == 0) return;
+    need(us && points_out, "null us or points_out");
+    PbDeviceGuard device_guard(c->device);
+    map_to_g2_impl(c, us, n, points_out);
+  });
+}
+
+int pb254_hash_to_g2(pb254_ctx* c, const uint64_t* messages, size_t n, size_t msg_len, uint64_t seed,
+                     uint64_t* inputs_out, uint64_t* hashes_out) {
+  return guarded([&] {
+    need_ctx(c);
+    need(n <= h2g2::MAX_N, "more than 2^17 messages");
+    need(msg_len <= h2g2::MAX_MSG_ELEMS && n * msg_len <= h2g2::MAX_MSG_ELEMS, "more than 2^24 message elements");
+    if (n == 0) return;
+    need((messages || msg_len == 0) && inputs_out && hashes_out, "null messages, inputs_out or hashes_out");
+    PbDeviceGuard device_guard(c->device);
+    hash_to_g2_impl(c, messages, n, msg_len, seed, inputs_out, hashes_out);
   });
 }
 

@@ -350,6 +350,28 @@ class Context:
                                                         _p(sums)))
         return inputs, sums
 
+    def map_to_g2(self, us):
+        """pb254_map_to_g2: the SvdW map of ``workloads.map_to_curve``. us (n, 8) canonical words of u (c0, c1) in Fq2.
+        Returns (n, 16): x.c0, x.c1, y.c0, y.c1 of each point of the G2 curve."""
+        us = _u64(us).reshape(-1, 8)
+        out = np.empty((us.shape[0], 16), dtype=np.uint64)
+        self.L.check(self.L.lib.pb254_map_to_g2(self._h, _p(us), C.c_size_t(us.shape[0]), _p(out)))
+        return out
+
+    def hash_to_g2(self, messages, seed: int):
+        """pb254_hash_to_g2 over messages (n, msg_len) canonical Goldilocks elements. Returns (inputs, hashes): inputs
+        (n, 36) the pb254_prove G2 rows (cofactor, map_to_g2(hash_to_fq2(m)), offset = k * G2 with k drawn from
+        SplitMix64(seed) as ``workloads.hash_to_g2_inputs`` draws it), hashes (n, 16) cofactor * x, the hash_to_g2
+        outputs."""
+        m = _u64(messages)
+        if m.ndim != 2:
+            raise Pb254Error(6, "messages must be (n, msg_len)")
+        inputs = np.empty((m.shape[0], 36), dtype=np.uint64)
+        hashes = np.empty((m.shape[0], 16), dtype=np.uint64)
+        self.L.check(self.L.lib.pb254_hash_to_g2(self._h, _p(m), C.c_size_t(m.shape[0]), C.c_size_t(m.shape[1]),
+                                                 C.c_uint64(seed & (2**64 - 1)), _p(inputs), _p(hashes)))
+        return inputs, hashes
+
     # ---- proving --------------------------------------------------------------------------
     def prove(self, kind, inputs, timestamps, min_rows=1 << 16, config: Config | None = None, keep_debug=False):
         """generate_trace + prove on the device; returns a :class:`Proof`."""

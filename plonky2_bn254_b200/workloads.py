@@ -9,7 +9,8 @@ reference that produce large batches of hot-path work items.
   y^2 = x^3 + 3/(9+u) -> cofactor clearing, which the circuit does as ``g2_scalar_mul(cofactor, point, offset)``
   with a random offset (:195-208) followed by ``- offset``. A batch of messages is a batch of
   ``G2ScalarMulInput {s: cofactor, x: mapped point, offset}``; ``hash_to_g2_outputs`` removes the offsets from the
-  STARK's native results.
+  STARK's native results. ``hash_to_g2_inputs_device`` builds the same batch, and the hashes, on the device
+  (``Context.hash_to_g2``).
 * ``g1_msm`` (src/utils/g1_msm.rs:22-36): a chain of G1 scalar-muls threaded through ``offset`` from a random subgroup
   point; ``g1_msm_inputs`` builds the batch on the device (``Context.scalar_mul_chains``) and returns the MSM.
 
@@ -221,6 +222,16 @@ def hash_to_g2_inputs(messages, permute, seed: int):
         offsets.append(off)
         rows.append(I._words(G2_COFACTOR) + _g2_words(pt) + _g2_words(off))
     return (np.array(rows, dtype=np.uint64).reshape(len(rows), 36), np.arange(len(rows), dtype=np.uint64), offsets)
+
+
+def hash_to_g2_inputs_device(ctx, messages, seed: int):
+    """``hash_to_g2_inputs`` built on the device (``Context.hash_to_g2``): the same rows whenever no drawn k is 0 mod r
+    (the device fails with E_BAD_ARG where Python would draw again, probability about 2^-253 per message).
+    Returns (inputs[n, 36], timestamps[n], offsets, hashes); offsets and hashes are affine points (x, y) of Fq2 pairs,
+    so that ``hash_to_g2_outputs(results, offsets)`` applies unchanged, and hashes[i] is the hash_to_g2 output."""
+    inputs, hashes = ctx.hash_to_g2(messages, seed)
+    offsets = [_g2_from_words(r[20:36]) for r in inputs]
+    return inputs, np.arange(inputs.shape[0], dtype=np.uint64), offsets, [_g2_from_words(h) for h in hashes]
 
 
 def hash_to_g2_outputs(results, offsets):

@@ -118,6 +118,9 @@ extern "C" {
     pub fn pb254_scalar_mul_chains(ctx: *mut pb254_ctx, kind: c_int, terms: *const u64, n_terms: usize,
                                    chain_starts: *const u64, n_chains: usize, offsets: *const u64,
                                    inputs_out: *mut u64, sums_out: *mut u64) -> c_int;
+    pub fn pb254_map_to_g2(ctx: *mut pb254_ctx, us: *const u64, n: usize, points_out: *mut u64) -> c_int;
+    pub fn pb254_hash_to_g2(ctx: *mut pb254_ctx, messages: *const u64, n: usize, msg_len: usize, seed: u64,
+                            inputs_out: *mut u64, hashes_out: *mut u64) -> c_int;
     pub fn pb254_prove(ctx: *mut pb254_ctx, kind: c_int, inputs: *const u64, timestamps: *const u64, n_inputs: usize,
                        min_rows: usize, cfg: *const pb254_config, keep_debug: c_int, out: *mut *mut pb254_proof) -> c_int;
     pub fn pb254_prove_dev(ctx: *mut pb254_ctx, kind: c_int, d_inputs: *const u64, d_timestamps: *const u64,

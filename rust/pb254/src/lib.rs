@@ -190,6 +190,39 @@ impl Context {
         Ok((inputs, sums))
     }
 
+    /// `pb254_map_to_g2`: the SvdW map of `HashToG2::map_to_g2` (src/utils/hash_to_g2.rs:113-147) before cofactor
+    /// clearing. `us` holds n values u in Fq2, 8 words each (c0, c1); returns n affine points of the G2 curve, 16 words
+    /// each (x.c0, x.c1, y.c0, y.c1).
+    pub fn map_to_g2(&self, us: &[u64]) -> Result<Vec<u64>> {
+        if us.len() % 8 != 0 {
+            return Err(anyhow!("map_to_g2: {} words are not whole Fq2 values", us.len()));
+        }
+        let n = us.len() / 8;
+        let mut points = vec![0u64; n * 16];
+        check(unsafe { sys::pb254_map_to_g2(self.0, us.as_ptr(), n, points.as_mut_ptr()) })?;
+        Ok(points)
+    }
+
+    /// `pb254_hash_to_g2`: `HashToG2::hash_to_g2` (src/utils/hash_to_g2.rs:76-148) of `n` equally long messages of
+    /// canonical Goldilocks elements, concatenated in `messages` (empty messages are valid), with the circuit's
+    /// cofactor clearing (:195-208). Returns (inputs, hashes): the `pack_g2` rows (cofactor, mapped point, offset
+    /// k_i G2 with k_i drawn from SplitMix64(seed)), ready for `prove`, and the n hash_to_g2 outputs (16 words each).
+    pub fn hash_to_g2(&self, messages: &[u64], n: usize, seed: u64) -> Result<(Vec<u64>, Vec<u64>)> {
+        if n == 0 {
+            return Ok((Vec::new(), Vec::new()));
+        }
+        if messages.len() % n != 0 {
+            return Err(anyhow!("hash_to_g2: {} words are not {} equally long messages", messages.len(), n));
+        }
+        let msg_len = messages.len() / n;
+        let mut inputs = vec![0u64; n * 36];
+        let mut hashes = vec![0u64; n * 16];
+        check(unsafe {
+            sys::pb254_hash_to_g2(self.0, messages.as_ptr(), n, msg_len, seed, inputs.as_mut_ptr(), hashes.as_mut_ptr())
+        })?;
+        Ok((inputs, hashes))
+    }
+
     /// The G1ScalarMulInput batch of `g1_msm(scalars, points)` (src/utils/g1_msm.rs:22-36) as one chain from a
     /// random subgroup point `offset`: returns (the `pack_g1` words of the batch, sum s_i x_i), the MSM being
     /// acc_N - acc_0. An accumulator at infinity is an error, as in the reference (g1_msm.rs:20-21).
