@@ -200,7 +200,7 @@ int pb254_prove_trace(pb254_ctx* ctx, int kind, const uint64_t* trace_cols, size
                       int keep_debug, pb254_proof** out);
 void pb254_proof_free(pb254_proof* proof);
 
-/* ---- verification (host; the reference verifies on the CPU as well) ----------------------------- */
+/* ---- verification (pb254_verify on the host, as the reference; pb254_verify_device on a context) ---- */
 /* verify(stark, config, ctls, proof, public_inputs = [], extra_looking_values)
  * (src/starks/common/verifier.rs:32-98) on a serialized proof. As in the reference, the STARK (`kind`) and the
  * StarkConfig (`cfg`, NULL = standard_fast_config) are the CALLER's: a proof whose header names another kind or
@@ -211,6 +211,13 @@ void pb254_proof_free(pb254_proof* proof);
  * (pb254_last_error() names the failed check). Needs no context and no GPU. */
 int pb254_verify(int kind, const pb254_config* cfg, const uint64_t* proof_words, size_t n_words,
                  const uint64_t* inputs, const uint64_t* timestamps, size_t n_inputs);
+/* pb254_verify with the native CTL values and all Merkle openings computed on the context's GPU. Same arguments
+ * and the same result as pb254_verify: for every input it returns the same code and pb254_last_error() names the
+ * same failed check. PB254_E_CUDA / PB254_E_OOM are the only additional outcomes. The transcript, the quotient
+ * identity at zeta and the FRI folds run on the calling thread; stage times are "verify native ctl" and
+ * "verify merkle" (pb254_timing_*). */
+int pb254_verify_device(pb254_ctx* ctx, int kind, const pb254_config* cfg, const uint64_t* proof_words,
+                        size_t n_words, const uint64_t* inputs, const uint64_t* timestamps, size_t n_inputs);
 /* Serialized StarkProofWithMetadata: little-endian u64 words, field order of SURVEY.md C.7 behind a
  * 10-word header {magic, kind, degree_bits, config[7]} (layout in DESIGN.md). */
 size_t pb254_proof_words(const pb254_proof* proof);

@@ -14,6 +14,7 @@ std::atomic<unsigned long long> g_pb_launches{0};
 #include "hash_to_g2.cuh"
 #include "prover.cuh"
 #include "verify.cuh"
+#include "verify_dev.cuh"
 
 struct pb254_proof {
   prover::ProofData data;
@@ -824,6 +825,21 @@ int pb254_verify(int kind, const pb254_config* cfg_in, const uint64_t* proof_wor
     need(proof_words && inputs && timestamps, "null argument");
     const pb254_config cfg = config_or_default(cfg_in, -1);
     verify::verify_proof(kind, cfg, proof_words, n_words, inputs, timestamps, n_inputs);
+  });
+}
+
+// pb254_verify with the native CTL values and the Merkle openings on the context's GPU (verify_dev.cuh): the same walk,
+// so the same code and message for every input; PB254_E_CUDA / PB254_E_OOM are the only additional outcomes.
+int pb254_verify_device(pb254_ctx* c, int kind, const pb254_config* cfg_in, const uint64_t* proof_words,
+                        size_t n_words, const uint64_t* inputs, const uint64_t* timestamps, size_t n_inputs) {
+  return guarded([&] {
+    need_ctx(c);
+    need_kind(kind);
+    need(proof_words && inputs && timestamps, "null argument");
+    const pb254_config cfg = config_or_default(cfg_in, -1);
+    PbDeviceGuard device_guard(c->device);
+    verify_dev::DeviceChecks checks(c);
+    verify::verify_walk(kind, cfg, proof_words, n_words, inputs, timestamps, n_inputs, checks);
   });
 }
 

@@ -5,12 +5,16 @@
 //   verify_stark_proof_with_challenges, verify_fri_proof   starky 0.4.0 / plonky2 0.2.2 (un-vendored)
 // and evaluates the constraint system at zeta in the quadratic extension in the emission order of
 //   eval_ext_circuit's native twin eval_packed_generic (SURVEY.md Appendix D).
-// The reference verifies on the CPU (milliseconds); so does this: verification is not part of the prover
-// hot path and touches kilobytes. Everything here is plain host C++ over gl:: / poseidon:: / bn:: helpers.
+// One walk (verify_walk) runs the checks in the reference's order. Its two heavy parts come from a Checks provider:
+// the native CTL values (one scalar multiplication, or x^s, per instance: 0.2 - 2.3 s serially at the BASELINE sizes,
+// profiles/r1_configs.md) and the Merkle openings of every query. HostChecks computes them here on the CPU
+// (pb254_verify); verify_dev.cuh computes them on the context's GPU (pb254_verify_device). The per-instance native
+// output and the Merkle path walk are PB_HD and shared by both, so both report the same error for every input.
+// The transcript, the quotient identity at zeta and the FRI folds stay on the host.
 #pragma once
 #include "../../include/pb254.h"
 #include "prover.cuh"
-#include "bn254.cuh"
+#include "chains.cuh"
 #include <vector>
 
 namespace verify {
@@ -294,14 +298,28 @@ static inline void eval_all(Consumer& y, int kind, const Rows& R, const aux::Cha
 }
 
 // ---- native CTL tuples (g1_generate_ctl_values and analogues) --------------------------------------
+// Per-instance outcome of the native computation (host and device): NATIVE_OK or the first failed check.
+enum { NATIVE_OK, NATIVE_NOT_CANONICAL, NATIVE_ORDER_TWO, NATIVE_INTERMEDIATE_INF, NATIVE_RESULT_INF };
+static inline Pb254Error native_error(int status) {
+  switch (status) {
+    case NATIVE_NOT_CANONICAL: return Pb254Error(PB254_E_NOT_CANONICAL, "input coordinate >= p");
+    case NATIVE_ORDER_TWO: return Pb254Error(PB254_E_INFINITY, "native result: point of order two");
+    case NATIVE_INTERMEDIATE_INF: return Pb254Error(PB254_E_INFINITY, "native result: intermediate point at infinity");
+    default: return Pb254Error(PB254_E_INFINITY, "native result: s * x + offset is the point at infinity");
+  }
+}
+
+// r = s * x + off by double-and-add from the top bit of s, as g1_generate_ctl_values computes it; x need not lie in
+// the prime-order subgroup (hash_to_g2 rows). Returns NATIVE_OK or the NATIVE_* infinity that stopped the ladder.
 template <class F>
-static inline bn::Aff<F> native_scalar_mul(const u64 s[4], const bn::Aff<F>& x, const bn::Aff<F>& off) {
+PB_HD int native_scalar_mul(const u64* s, const bn::Aff<F>& x, const bn::Aff<F>& off, bn::Aff<F>& r) {
   bn::Jac<F> acc;
   bool started = false;
   int st = 0;
+#pragma unroll 1
   for (int j = 255; j >= 0; j--) {
     if (started) {
-      if (F::is_zero(acc.Y)) throw Pb254Error(PB254_E_INFINITY, "native result: point of order two");
+      if (F::is_zero(acc.Y)) return NATIVE_ORDER_TWO;
       acc = bn::jac_double<F>(acc);
     }
     if ((s[j >> 6] >> (j & 63)) & 1) {
@@ -312,22 +330,36 @@ static inline bn::Aff<F> native_scalar_mul(const u64 s[4], const bn::Aff<F>& x, 
         started = true;
       } else {
         acc = bn::jac_add_mixed<F>(acc, x, st);
-        if (st == 2) throw Pb254Error(PB254_E_INFINITY, "native result: intermediate point at infinity");
+        if (st == 2) return NATIVE_INTERMEDIATE_INF;
       }
     }
   }
-  if (!started) return off;
+  if (!started) {
+    r = off;
+    return NATIVE_OK;
+  }
   acc = bn::jac_add_mixed<F>(acc, off, st);
-  if (st == 2) throw Pb254Error(PB254_E_INFINITY, "native result: s * x + offset is the point at infinity");
+  if (st == 2) return NATIVE_RESULT_INF;
   typename F::T zi = F::inv(acc.Z), zi2 = F::sqr(zi);
-  bn::Aff<F> r;
   r.x = F::mul(acc.X, zi2);
   r.y = F::mul(acc.Y, F::mul(zi, zi2));
-  return r;
+  return NATIVE_OK;
 }
 
-static inline bool words_canonical(const u64* w) {
-  static const u64 PW[4] = {0x3c208c16d87cfd47ULL, 0x97816a916871ca8dULL, 0xb85045b68181585dULL, 0x30644e72e131a029ULL};
+// x^s, square-and-multiply from bit 255 (fq_exp)
+PB_HD bn::Fq native_fq_exp(const u64* s, const bn::Fq& x) {
+  bn::Fq acc = bn::one();
+#pragma unroll 1
+  for (int j = 255; j >= 0; j--) {
+    acc = bn::sqr(acc);
+    if ((s[j >> 6] >> (j & 63)) & 1) acc = bn::mul(acc, x);
+  }
+  return acc;
+}
+
+PB_HD bool words_canonical(const u64* w) {
+  const u64 PW[4] = {0x3c208c16d87cfd47ULL, 0x97816a916871ca8dULL, 0xb85045b68181585dULL, 0x30644e72e131a029ULL};
+#pragma unroll
   for (int i = 3; i >= 0; i--) {
     if (w[i] < PW[i]) return true;
     if (w[i] > PW[i]) return false;
@@ -337,103 +369,197 @@ static inline bool words_canonical(const u64* w) {
 static inline void push_limbs(std::vector<u64>& out, const u64* w) {
   for (int i = 0; i < 16; i++) out.push_back((w[i >> 2] >> (16 * (i & 3))) & 0xffff);
 }
-static inline void push_fq_limbs(std::vector<u64>& out, const bn::Fq& mont) {
-  int lim[16];
-  bn::to_limbs16(bn::from_mont(mont), lim);
-  for (int i = 0; i < 16; i++) out.push_back((u64)lim[i]);
+// the Montgomery form of the canonical words at w; false if they are >= p
+PB_HD bool load_fq(const u64* w, bn::Fq& out) {
+  if (!words_canonical(w)) return false;
+  out = bn::to_mont(bn::from_words(w));
+  return true;
 }
-static inline bn::Fq load_fq(const u64* w) {
-  if (!words_canonical(w)) throw Pb254Error(PB254_E_NOT_CANONICAL, "input coordinate >= p");
-  return bn::to_mont(bn::from_words(w));
+
+// Canonical words of the native output of the input row w: x^s (4 words), s * x + offset in G1 (x, y: 8) or G2
+// (x.c0, x.c1, y.c0, y.c1: 16). Returns NATIVE_OK or the first failed check, in the order of the reference walk.
+template <int KIND>
+PB_HD int native_output(const u64* w, u64* out) {
+  if (KIND == 2) {
+    bn::Fq x;
+    if (!load_fq(w + 4, x)) return NATIVE_NOT_CANONICAL;
+    chains::put_fq(out, native_fq_exp(w, x));
+    return NATIVE_OK;
+  } else if (KIND == 0) {
+    bn::Aff<bn::F1> x, off, r;
+    if (!(load_fq(w + 4, x.x) & load_fq(w + 8, x.y) & load_fq(w + 12, off.x) & load_fq(w + 16, off.y)))
+      return NATIVE_NOT_CANONICAL;
+    const int st = native_scalar_mul<bn::F1>(w, x, off, r);
+    if (st) return st;
+    chains::put_fq(out, r.x);
+    chains::put_fq(out + 4, r.y);
+    return NATIVE_OK;
+  } else {
+    bn::Aff<bn::F2> x, off, r;
+    if (!(load_fq(w + 4, x.x.c0) & load_fq(w + 8, x.x.c1) & load_fq(w + 12, x.y.c0) & load_fq(w + 16, x.y.c1) &
+          load_fq(w + 20, off.x.c0) & load_fq(w + 24, off.x.c1) & load_fq(w + 28, off.y.c0) & load_fq(w + 32, off.y.c1)))
+      return NATIVE_NOT_CANONICAL;
+    const int st = native_scalar_mul<bn::F2>(w, x, off, r);
+    if (st) return st;
+    chains::put_fq(out, r.x.c0);
+    chains::put_fq(out + 4, r.x.c1);
+    chains::put_fq(out + 8, r.y.c0);
+    chains::put_fq(out + 12, r.y.c1);
+    return NATIVE_OK;
+  }
+}
+static inline int native_output(int kind, const u64* w, u64* out) {
+  return kind == 0 ? native_output<0>(w, out) : kind == 1 ? native_output<1>(w, out) : native_output<2>(w, out);
 }
 
 // tuples[0][k] = looked values of CTL 0 (inputs) for instance k, tuples[1][k] = CTL 1 (outputs)
 static inline void ctl_tuples(int kind, const u64* inputs, const u64* ts, size_t K, std::vector<std::vector<u64>> tuples[2]) {
   const tg::Layout l = tg::layout_for(kind);
+  const int out_words = kind == 0 ? 8 : kind == 1 ? 16 : 4;
   tuples[0].assign(K, {});
   tuples[1].assign(K, {});
-  // an exception must not leave an OpenMP region (hostsim build): remember the first one and rethrow afterwards
-  int err_code = 0;
-  std::string err_msg;
+  // the lowest failing instance's error is reported, also when the hostsim build runs this loop with OpenMP
+  size_t err_k = K;
+  int err_status = NATIVE_OK;
 #pragma omp parallel for schedule(dynamic, 4)
   for (long long kk = 0; kk < (long long)K; kk++) {
     const size_t k = (size_t)kk;
-    try {
     const u64* w = inputs + k * l.in_words;
     std::vector<u64>&in = tuples[0][k], &out = tuples[1][k];
-    if (kind == 2) {
-      push_limbs(in, w + 4);  // b = x
-      bn::Fq x = load_fq(w + 4), acc = bn::one();
-      for (int j = 255; j >= 0; j--) {
-        acc = bn::sqr(acc);
-        if ((w[j >> 6] >> (j & 63)) & 1) acc = bn::mul(acc, x);
+    u64 r[16];
+    const int st = native_output(kind, w, r);
+    if (st) {
+#pragma omp critical
+      if (k < err_k) {
+        err_k = k;
+        err_status = st;
       }
-      push_fq_limbs(out, acc);
-    } else if (kind == 0) {
-      for (int c = 0; c < 2; c++) push_limbs(in, w + 4 + 4 * c);       // x
-      for (int c = 0; c < 2; c++) push_limbs(in, w + 12 + 4 * c);      // offset
-      bn::Aff<bn::F1> x{load_fq(w + 4), load_fq(w + 8)}, off{load_fq(w + 12), load_fq(w + 16)};
-      bn::Aff<bn::F1> r = native_scalar_mul<bn::F1>(w, x, off);
-      push_fq_limbs(out, r.x);
-      push_fq_limbs(out, r.y);
-    } else {
-      for (int c = 0; c < 4; c++) push_limbs(in, w + 4 + 4 * c);
-      for (int c = 0; c < 4; c++) push_limbs(in, w + 20 + 4 * c);
-      bn::Aff<bn::F2> x{{load_fq(w + 4), load_fq(w + 8)}, {load_fq(w + 12), load_fq(w + 16)}};
-      bn::Aff<bn::F2> off{{load_fq(w + 20), load_fq(w + 24)}, {load_fq(w + 28), load_fq(w + 32)}};
-      bn::Aff<bn::F2> r = native_scalar_mul<bn::F2>(w, x, off);
-      push_fq_limbs(out, r.x.c0);
-      push_fq_limbs(out, r.x.c1);
-      push_fq_limbs(out, r.y.c0);
-      push_fq_limbs(out, r.y.c1);
+      continue;
     }
-    push_limbs(in, w);  // s as 16 limbs
+    for (int c = 4; c < l.in_words; c += 4) push_limbs(in, w + c);  // x (and the offset)
+    push_limbs(in, w);                                                // s as 16 limbs
+    for (int c = 0; c < out_words; c += 4) push_limbs(out, r + c);
     in.push_back(ts[k] % gl::P);
     out.push_back(ts[k] % gl::P);
-    } catch (const Pb254Error& e) {
-#pragma omp critical
-      if (!err_code) {
-        err_code = e.code;
-        err_msg = e.what();
-      }
-    }
   }
-  if (err_code) throw Pb254Error(err_code, err_msg);
+  if (err_status) throw native_error(err_status);
 }
 
 // ---- Merkle ------------------------------------------------------------------------------------------
-static inline Digest hash_or_noop(const u64* v, size_t n) {
-  Digest d;
+// hash_or_noop of the leaf v[0..n), then the path of `depth` siblings up to the cap entry; true if they agree. Every
+// word must be canonical (the walk has checked the whole blob): the device permutation requires canonical inputs.
+PB_HD void hash_or_noop(const u64* v, size_t n, u64 d[4]) {
   if (n <= 4) {
-    for (int i = 0; i < 4; i++) d.e[i] = (size_t)i < n ? v[i] : 0;
-    return d;
+#pragma unroll
+    for (int i = 0; i < 4; i++) d[i] = (size_t)i < n ? v[i] : 0;
+    return;
   }
-  u64 s[12] = {0};
+  u64 s[12];
+#pragma unroll
+  for (int i = 0; i < 12; i++) s[i] = 0;
+#pragma unroll 1
   for (size_t c = 0; c < n; c += 8) {
-    for (size_t k = 0; k < 8 && c + k < n; k++) s[k] = v[c + k];
+#pragma unroll
+    for (int k = 0; k < 8; k++)
+      if (c + k < n) s[k] = v[c + k];
     poseidon::permute(s);
   }
-  for (int i = 0; i < 4; i++) d.e[i] = s[i];
-  return d;
+#pragma unroll
+  for (int i = 0; i < 4; i++) d[i] = s[i];
 }
-static inline void check_merkle(const u64* leaf, size_t leaf_len, size_t index, const u64* siblings, int depth,
-                                const u64* cap, const char* what) {
-  Digest cur = hash_or_noop(leaf, leaf_len);
+PB_HD bool merkle_path_ok(const u64* leaf, size_t leaf_len, size_t index, const u64* siblings, int depth,
+                          const u64* cap) {
+  Digest cur;
+  hash_or_noop(leaf, leaf_len, cur.e);
+#pragma unroll 1
   for (int lv = 0; lv < depth; lv++) {
     Digest sib;
-    memcpy(sib.e, siblings + 4 * lv, 32);
-    cur = (index & 1) ? poseidon::two_to_one(sib, cur) : poseidon::two_to_one(cur, sib);
+#pragma unroll
+    for (int i = 0; i < 4; i++) sib.e[i] = siblings[4 * lv + i];
+    const bool right = index & 1;
+    cur = poseidon::two_to_one(right ? sib : cur, right ? cur : sib);
     index >>= 1;
   }
-  if (memcmp(cur.e, cap + 4 * index, 32) != 0) throw VerifyError(std::string("Merkle path of the ") + what);
+  bool same = true;
+#pragma unroll
+  for (int i = 0; i < 4; i++) same &= cur.e[i] == cap[4 * index + i];
+  return same;
 }
+
+// ---- the two heavy parts of verification -----------------------------------------------------------
+// What verify_walk knows once the transcript has run: the caller's batch, the proof and its layout, the CTL
+// challenges and the query indices.
+struct Job {
+  int kind, nch, logN, cap_h;
+  const u64* blob;
+  size_t words;
+  const pb254_proof_layout* lay;
+  const u64 *inputs, *timestamps;
+  size_t K;
+  const aux::Challenges* chal;
+  const std::vector<u64>* idx;
+  const std::vector<unsigned>* arities;
+};
+struct CtlResults {
+  int code = 0;               // the lowest failing instance's native error (0: none) ...
+  std::string msg;            // ... and its message
+  std::vector<uint8_t> zero;  // [c * nch + j]: some combination of CTL c under challenge j is zero
+  std::vector<u64> sum;       // [c * nch + j]: the sum of the inverses of those combinations
+};
+// Tree t of a query: 0 trace, 1 auxiliary, 2 quotient, 3 + i FRI layer i.
+struct Checks {
+  virtual ~Checks() {}
+  virtual void start(const Job& job) = 0;  // called once, before the quotient identity is evaluated
+  virtual void ctl(CtlResults& out) = 0;
+  virtual bool merkle_ok(size_t q, int tree, const u64* leaf, size_t leaf_len, size_t index, const u64* siblings,
+                         int depth, const u64* cap) = 0;
+};
+
+// pb254_verify: both parts computed here on the CPU, the Merkle paths when the walk asks for them
+struct HostChecks : Checks {
+  Job job;
+  void start(const Job& j) override { job = j; }
+  void ctl(CtlResults& o) override {
+    const int nch = job.nch;
+    std::vector<std::vector<u64>> tuples[2];
+    try {
+      ctl_tuples(job.kind, job.inputs, job.timestamps, job.K, tuples);
+    } catch (const Pb254Error& e) {
+      o.code = e.code;
+      o.msg = e.what();
+      return;
+    }
+    o.zero.assign(2 * nch, 0);
+    o.sum.assign(2 * nch, 0);
+    for (int c = 0; c < 2; c++)
+      for (int j = 0; j < nch; j++) {
+        u64 sum = 0;
+        for (size_t k = 0; k < job.K; k++) {
+          const std::vector<u64>& t = tuples[c][k];
+          u64 comb = 0;
+          for (size_t i = t.size(); i-- > 0;) comb = gl::add(gl::mul(comb, job.chal->beta[j]), t[i]);
+          comb = gl::add(comb, job.chal->gamma[j]);
+          if (comb == 0) {
+            o.zero[c * nch + j] = 1;
+            break;
+          }
+          sum = gl::add(sum, gl::inv(comb));
+        }
+        o.sum[c * nch + j] = sum;
+      }
+  }
+  bool merkle_ok(size_t, int, const u64* leaf, size_t leaf_len, size_t index, const u64* siblings, int depth,
+                 const u64* cap) override {
+    return merkle_path_ok(leaf, leaf_len, index, siblings, depth, cap);
+  }
+};
 
 // ---- the verifier -------------------------------------------------------------------------------------
 // `kind` and `cfg` are the CALLER's (the reference's verify(stark, config, ...) takes the StarkConfig from the caller,
 // src/starks/common/verifier.rs:32-45): every security parameter stamped into the blob header must equal them, only
 // degree_bits is read from the proof. `inputs` holds K rows of in_words(kind) words.
-static inline void verify_proof(int kind, const pb254_config& cfg, const u64* blob, size_t words, const u64* inputs,
-                                const u64* timestamps, size_t K) {
+static inline void verify_walk(int kind, const pb254_config& cfg, const u64* blob, size_t words, const u64* inputs,
+                               const u64* timestamps, size_t K, Checks& checks) {
   if (kind < 0 || kind > 2) throw Pb254Error(PB254_E_BAD_ARG, "unknown STARK kind");
   prover::validate_config(cfg);
   if (words < 22 || blob[0] != prover::PROOF_MAGIC) throw VerifyError("not a pb254 proof blob");
@@ -515,6 +641,10 @@ static inline void verify_proof(int kind, const pb254_config& cfg, const u64* bl
   if (cfg.pow_bits && (pow_resp >> (64 - cfg.pow_bits)) != 0) throw VerifyError("proof of work");
   std::vector<u64> idx(nq);
   for (auto& x : idx) x = ch.challenge() % (u64)N;
+  {
+    const Job job{kind, nch, logN, cap_h, blob, words, &lay, inputs, timestamps, K, &chal, &idx, &arities};
+    checks.start(job);
+  }
 
   // ---- quotient identity at zeta -------------------------------------------------------------------
   const u64 g = gl::root_of_unity(L);
@@ -544,20 +674,13 @@ static inline void verify_proof(int kind, const pb254_config& cfg, const u64* bl
 
   // ---- cross-table lookup sums (verifier.rs:88-95, ctl_values.rs:28-47) ----------------------------
   {
-    std::vector<std::vector<u64>> tuples[2];
-    ctl_tuples(kind, inputs, timestamps, K, tuples);
+    CtlResults ctl;
+    checks.ctl(ctl);
+    if (ctl.code) throw Pb254Error(ctl.code, ctl.msg);
     for (int c = 0; c < 2; c++)
       for (int j = 0; j < nch; j++) {
-        u64 sum = 0;
-        for (size_t k = 0; k < K; k++) {
-          const std::vector<u64>& t = tuples[c][k];
-          u64 comb = 0;
-          for (size_t i = t.size(); i-- > 0;) comb = gl::add(gl::mul(comb, chal.beta[j]), t[i]);
-          comb = gl::add(comb, chal.gamma[j]);
-          if (comb == 0) throw VerifyError("CTL combination is zero");
-          sum = gl::add(sum, gl::inv(comb));
-        }
-        if (sum != zs_first[c * nch + j]) throw VerifyError("cross-table lookup sum");
+        if (ctl.zero[c * nch + j]) throw VerifyError("CTL combination is zero");
+        if (ctl.sum[c * nch + j] != zs_first[c * nch + j]) throw VerifyError("cross-table lookup sum");
       }
   }
 
@@ -584,9 +707,12 @@ static inline void verify_proof(int kind, const pb254_config& cfg, const u64* bl
     size_t x_index = (size_t)idx[q];
     const u64 *row_tr = rp, *sib_tr = rp + W, *row_ax = sib_tr + nsib, *sib_ax = row_ax + A, *row_q = sib_ax + nsib,
               *sib_q = row_q + Q;
-    check_merkle(row_tr, W, x_index, sib_tr, logN - cap_h, caps, "trace tree");
-    check_merkle(row_ax, A, x_index, sib_ax, logN - cap_h, caps + capw, "auxiliary tree");
-    check_merkle(row_q, Q, x_index, sib_q, logN - cap_h, caps + 2 * capw, "quotient tree");
+    if (!checks.merkle_ok(q, 0, row_tr, W, x_index, sib_tr, logN - cap_h, caps))
+      throw VerifyError("Merkle path of the trace tree");
+    if (!checks.merkle_ok(q, 1, row_ax, A, x_index, sib_ax, logN - cap_h, caps + capw))
+      throw VerifyError("Merkle path of the auxiliary tree");
+    if (!checks.merkle_ok(q, 2, row_q, Q, x_index, sib_q, logN - cap_h, caps + 2 * capw))
+      throw VerifyError("Merkle path of the quotient tree");
     const u64 x = gl::mul(gl::COSET_SHIFT, gl::pow(wN, gl::brev32((u32)x_index, logN)));
     E2 f0 = X(0), f1 = X(0), f2 = X(0);
     for (int c = 0; c < W; c++) f1 = f1 + gl::emul_base(apow[c], row_tr[c]);
@@ -609,7 +735,8 @@ static inline void verify_proof(int kind, const pb254_config& cfg, const u64* bl
       const u64* sib = lp + 2 * arity;
       const size_t coset = x_index >> ab, within = x_index & (size_t)(arity - 1);
       if (!(gl::e2(evals[2 * within], evals[2 * within + 1]) == cur)) throw VerifyError("FRI layer consistency");
-      check_merkle(evals, 2 * (size_t)arity, coset, sib, log_leaves - cap_h, fri_caps + li * capw, "FRI layer tree");
+      if (!checks.merkle_ok(q, 3 + (int)li, evals, 2 * (size_t)arity, coset, sib, log_leaves - cap_h, fri_caps + li * capw))
+        throw VerifyError("Merkle path of the FRI layer tree");
       // fold (same formula as fri::FoldK)
       const u64 x0inv = gl::mul(gl::inv(shift), gl::pow(gl::inv(gl::root_of_unity(log_len)),
                                                          gl::brev32((u32)coset, log_leaves)));
@@ -640,6 +767,12 @@ static inline void verify_proof(int kind, const pb254_config& cfg, const u64* bl
     for (size_t i = keep; i-- > 0;) ev = gl::emul_base(ev, xf) + gl::e2(final_poly[2 * i], final_poly[2 * i + 1]);
     if (!(ev == cur)) throw VerifyError("FRI final polynomial");
   }
+}
+
+static inline void verify_proof(int kind, const pb254_config& cfg, const u64* blob, size_t words, const u64* inputs,
+                                const u64* timestamps, size_t K) {
+  HostChecks host;
+  verify_walk(kind, cfg, blob, words, inputs, timestamps, K, host);
 }
 
 }  // namespace verify

@@ -136,14 +136,18 @@ class Library:
     def verify(self, kind, proof_words, inputs, timestamps, config: "Config | None" = None) -> bool:
         """pb254_verify(kind, config, ...): True, or raises Pb254Error(E_VERIFY / ...) naming the failed check.
         `kind` and `config` (None = standard_fast_config) are the verifier's own, never the proof's."""
+        w, inputs, timestamps = self._verify_args(kind, proof_words, inputs, timestamps)
+        self.check(self.lib.pb254_verify(C.c_int(kind), C.byref(config) if config is not None else None, _p(w),
+                                         C.c_size_t(w.size), _p(inputs), _p(timestamps), C.c_size_t(inputs.shape[0])))
+        return True
+
+    def _verify_args(self, kind, proof_words, inputs, timestamps):
         w = _u64(proof_words)
         inputs = _u64(inputs)
         timestamps = _u64(timestamps)
         if inputs.ndim != 2 or inputs.shape[1] != self.input_words(kind) or timestamps.size != inputs.shape[0]:
             raise Pb254Error(6, "inputs must be (n, input_words(kind)) with one timestamp per row")
-        self.check(self.lib.pb254_verify(C.c_int(kind), C.byref(config) if config is not None else None, _p(w),
-                                         C.c_size_t(w.size), _p(inputs), _p(timestamps), C.c_size_t(inputs.shape[0])))
-        return True
+        return w, inputs, timestamps
 
 
     def parse_proof(self, proof_words) -> "ProofView":
@@ -384,6 +388,16 @@ class Context:
                                             C.byref(config) if config is not None else None, C.c_int(int(keep_debug)),
                                             C.byref(h)))
         return Proof(self.L, h)
+
+    def verify(self, kind, proof_words, inputs, timestamps, config: Config | None = None) -> bool:
+        """pb254_verify_device: :meth:`Library.verify` with the native CTL values and the Merkle openings computed on
+        this context's GPU. Same checks, same outcome for every input: True, or raises the same Pb254Error."""
+        w, inputs, timestamps = self.L._verify_args(kind, proof_words, inputs, timestamps)
+        self.L.check(self.L.lib.pb254_verify_device(self._h, C.c_int(kind),
+                                                    C.byref(config) if config is not None else None, _p(w),
+                                                    C.c_size_t(w.size), _p(inputs), _p(timestamps),
+                                                    C.c_size_t(inputs.shape[0])))
+        return True
 
     def prove_sharded(self, kind, inputs, timestamps, rank: int, world: int, all_to_all, all_gather,
                       min_rows=1 << 16, config: Config | None = None):

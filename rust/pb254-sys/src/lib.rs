@@ -137,6 +137,8 @@ extern "C" {
     pub fn pb254_proof_free(proof: *mut pb254_proof);
     pub fn pb254_verify(kind: c_int, cfg: *const pb254_config, proof_words: *const u64, n_words: usize,
                         inputs: *const u64, timestamps: *const u64, n_inputs: usize) -> c_int;
+    pub fn pb254_verify_device(ctx: *mut pb254_ctx, kind: c_int, cfg: *const pb254_config, proof_words: *const u64,
+                               n_words: usize, inputs: *const u64, timestamps: *const u64, n_inputs: usize) -> c_int;
     pub fn pb254_proof_parse(proof_words: *const u64, n_words: usize, out: *mut pb254_proof_layout) -> c_int;
     pub fn pb254_proof_results_words(proof: *const pb254_proof) -> usize;
     pub fn pb254_proof_results_data(proof: *const pb254_proof) -> *const u64;

@@ -305,6 +305,16 @@ impl Context {
         })?;
         Self::take(h)
     }
+
+    /// `verify` with the native CTL values and the Merkle openings computed on this context's GPU
+    /// (`pb254_verify_device`): the same checks in the same order, so the same result and error for every input.
+    pub fn verify(&self, kind: i32, config: Option<&StarkConfig>, blob: &[u64], words: &[u64], timestamps: &[u64]) -> Result<()> {
+        let cfg = config.map(config_of).transpose()?;
+        check(unsafe {
+            sys::pb254_verify_device(self.0, kind, cfg.as_ref().map_or(std::ptr::null(), |c| c as *const _), blob.as_ptr(),
+                                     blob.len(), words.as_ptr(), timestamps.as_ptr(), timestamps.len())
+        })
+    }
 }
 impl Drop for Context {
     fn drop(&mut self) {
