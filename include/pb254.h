@@ -268,8 +268,11 @@ int pb254_proof_parse(const uint64_t* proof_words, size_t n_words, pb254_proof_l
  * helpers chain them (src/utils/g1_msm.rs:22-36). Only filled by pb254_prove / pb254_prove_dev. */
 size_t pb254_proof_results_words(const pb254_proof* proof);
 const uint64_t* pb254_proof_results_data(const pb254_proof* proof);
-/* intermediate artefacts for parity tests (only when keep_debug != 0): which = 0 auxiliary values
- * (A x n), 1 quotient chunk coefficients (2*num_challenges x n), 2 challenges, 3 query indices */
+/* intermediate artefacts for parity tests: which = 0 auxiliary values (A x n), 1 quotient chunk coefficients
+ * (2*num_challenges x n), 2 challenges [betas, gammas, alphas, zeta, fri_alpha, fri_betas], 3 query indices,
+ * 5 the running quotient total of challenge 0 after every constraint group at quotient point 5 (64 words per pass of
+ * the quotient kernel, 4096 words). Slots 0-2 and 5 are filled only when keep_debug != 0, slot 3 always; any other
+ * `which` gives 0 words and NULL. */
 size_t pb254_proof_debug_words(const pb254_proof* proof, int which);
 const uint64_t* pb254_proof_debug_data(const pb254_proof* proof, int which);
 

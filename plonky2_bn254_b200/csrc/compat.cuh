@@ -123,6 +123,13 @@ struct PbDeviceGuard {
   PbDeviceGuard(const PbDeviceGuard&) = delete;
   PbDeviceGuard& operator=(const PbDeviceGuard&) = delete;
 };
+// free memory of device d (bytes)
+static inline size_t pb_free_bytes(int d) {
+  PbDeviceGuard device_guard(d);
+  size_t free_b = 0, total_b = 0;
+  PB_CUDA(cudaMemGetInfo(&free_b, &total_b));
+  return free_b;
+}
 
 // launch counter (reported by bench.py as gpu_launches)
 extern std::atomic<unsigned long long> g_pb_launches;

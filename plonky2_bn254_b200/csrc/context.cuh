@@ -50,6 +50,10 @@ struct StageTimes {
   };
   std::vector<Rec> recs;
   bool enabled = true;
+  StageTimes() = default;
+  ~StageTimes() { clear(); }  // the events belong to this object: no copies
+  StageTimes(const StageTimes&) = delete;
+  StageTimes& operator=(const StageTimes&) = delete;
 #if PB_HOSTSIM
   static double now() {
     struct timespec ts;

@@ -7,6 +7,7 @@
 std::atomic<unsigned long long> g_pb_launches{0};
 #include "context.cuh"
 #include "ntt.cuh"
+#include <memory>
 #include <thread>
 #include "merkle.cuh"
 #include "tracegen.h"
@@ -38,6 +39,21 @@ int guarded(F&& f) {
   }
 }
 
+// Every call on a context runs its work in this scope, after its argument checks: on the context's device, with an
+// empty arena of at least `arena_bytes` and an empty stage list. A call that succeeds drains the stream and reads the
+// stage times. One that fails returns without waiting: a failed sharded proof may have left a collective in the stream
+// that the other ranks never enqueue.
+template <class F>
+void on_context(pb254_ctx* c, size_t arena_bytes, F&& body) {
+  PbDeviceGuard device_guard(c->device);
+  c->arena.reserve(arena_bytes);
+  c->arena.reset();
+  c->times.clear();
+  body();
+  pb_sync(c->stream);
+  c->times.resolve();
+}
+
 int ilog2_strict(size_t n) {
   int k = 0;
   while (((size_t)1 << k) < n) k++;
@@ -50,7 +66,8 @@ void need(bool ok, const char* what) {
   if (!ok) throw Pb254Error(PB254_E_BAD_ARG, what);
 }
 void need_ctx(const pb254_ctx* c) { need(c != nullptr, "null context"); }
-void need_kind(int kind) { need(kind >= 0 && kind <= 2, "unknown STARK kind (0 = G1, 1 = G2, 2 = Fq)"); }
+bool valid_kind(int kind) { return kind >= 0 && kind <= 2; }
+void need_kind(int kind) { need(valid_kind(kind), "unknown STARK kind (0 = G1, 1 = G2, 2 = Fq)"); }
 // trace heights: a power of two, at least 2^16 (the range-check table needs 65536 rows) and at most 2^26
 int need_trace_rows(size_t n_rows) {
   int k = 0;
@@ -67,18 +84,6 @@ pb254_config config_or_default(const pb254_config* cfg_in, int log_rows) {
   prover::validate_config(cfg);
   if (log_rows >= 0) need(cfg.cap_height <= (unsigned)log_rows + cfg.rate_bits, "cap_height larger than log2 of the LDE size");
   return cfg;
-}
-
-struct Shape {
-  int L, width, aux_len, in_words;
-};
-Shape shape_for(int kind) {
-  switch (kind) {
-    case PB254_KIND_G1: return {32, 781, 354, 20};
-    case PB254_KIND_G2: return {64, 1295, 708, 36};
-    case PB254_KIND_FQ: return {16, 427, 80, 8};
-  }
-  throw Pb254Error(PB254_E_BAD_ARG, "unknown STARK kind");
 }
 
 void throw_trace_error(int herr) {
@@ -131,7 +136,6 @@ void run_chains(pb254_ctx* c, const u64* d_terms, const u64* d_starts, const u64
   pb_d2h(&herr, B.err, sizeof(int), s);
   pb_d2h(&first_inf, B.first_inf, sizeof(unsigned), s);
   pb_sync(s);
-  c->times.resolve();
   if (herr == tg::ERR_NOT_CANONICAL || herr == tg::ERR_NOT_ON_CURVE) throw_trace_error(herr);
   if (first_inf != chains::NO_INF) {
     // element e = i + ch + 1 holds the accumulator after term i of chain ch
@@ -146,27 +150,27 @@ void run_chains(pb254_ctx* c, const u64* d_terms, const u64* d_starts, const u64
   throw_trace_error(herr);
   if (n_terms && inputs_out) pb_d2h(inputs_out, d_rows, n_terms * RW * 8, s);
   if (sums_out) pb_d2h(sums_out, d_sums, n_chains * 2 * FW * 8, s);
-  pb_sync(s);
 }
 
 template <class F>
 void scalar_mul_chains_impl(pb254_ctx* c, const u64* terms, size_t n_terms, const u64* chain_starts, size_t n_chains,
                             const u64* offsets, u64* inputs_out, u64* sums_out) {
   const size_t FW = tg::FieldIO<F>::WORDS, TW = 4 + 2 * FW, RW = TW + 2 * FW;
-  c->arena.reserve(chains::scratch_bytes<F>(n_terms, n_chains) +
-                   (n_terms * (TW + RW) + (n_chains + 1) + 2 * n_chains * 2 * FW) * 8 + 65536);
-  c->arena.reset();
-  c->times.clear();
-  const pbStream s = c->stream;
-  u64* d_terms = c->arena.alloc_n<u64>(n_terms * TW);
-  u64* d_starts = c->arena.alloc_n<u64>(n_chains + 1);
-  u64* d_offsets = c->arena.alloc_n<u64>(n_chains * 2 * FW);
-  u64* d_rows = c->arena.alloc_n<u64>(n_terms * RW);
-  u64* d_sums = sums_out ? c->arena.alloc_n<u64>(n_chains * 2 * FW) : nullptr;
-  if (n_terms) pb_h2d(d_terms, terms, n_terms * TW * 8, s);
-  pb_h2d(d_starts, chain_starts, (n_chains + 1) * 8, s);
-  pb_h2d(d_offsets, offsets, n_chains * 2 * FW * 8, s);
-  run_chains<F>(c, d_terms, d_starts, d_offsets, n_terms, chain_starts, n_chains, d_rows, d_sums, inputs_out, sums_out);
+  const size_t bytes = chains::scratch_bytes<F>(n_terms, n_chains) +
+                       (n_terms * (TW + RW) + (n_chains + 1) + 2 * n_chains * 2 * FW) * 8 + 65536;
+  on_context(c, bytes, [&] {
+    const pbStream s = c->stream;
+    u64* d_terms = c->arena.alloc_n<u64>(n_terms * TW);
+    u64* d_starts = c->arena.alloc_n<u64>(n_chains + 1);
+    u64* d_offsets = c->arena.alloc_n<u64>(n_chains * 2 * FW);
+    u64* d_rows = c->arena.alloc_n<u64>(n_terms * RW);
+    u64* d_sums = sums_out ? c->arena.alloc_n<u64>(n_chains * 2 * FW) : nullptr;
+    if (n_terms) pb_h2d(d_terms, terms, n_terms * TW * 8, s);
+    pb_h2d(d_starts, chain_starts, (n_chains + 1) * 8, s);
+    pb_h2d(d_offsets, offsets, n_chains * 2 * FW * 8, s);
+    run_chains<F>(c, d_terms, d_starts, d_offsets, n_terms, chain_starts, n_chains, d_rows, d_sums, inputs_out,
+                  sums_out);
+  });
 }
 
 // the lowest failing message (or u) of each h2g2::BAD_* slot, checked in stage order
@@ -192,26 +196,23 @@ void check_h2g2(pb254_ctx* c, const unsigned* d_bad) {
 }
 
 void map_to_g2_impl(pb254_ctx* c, const u64* us, size_t n, u64* points_out) {
-  c->arena.reserve(n * (8 * 8 + sizeof(h2g2::Fq2) + sizeof(h2g2::Aff) + 16 * 8) + 65536);
-  c->arena.reset();
-  c->times.clear();
-  const pbStream s = c->stream;
-  u64* d_us = c->arena.alloc_n<u64>(n * 8);
-  h2g2::Fq2* d_u = c->arena.alloc_n<h2g2::Fq2>(n);
-  h2g2::Aff* d_pts = c->arena.alloc_n<h2g2::Aff>(n);
-  u64* d_out = c->arena.alloc_n<u64>(n * 16);
-  unsigned* d_bad = c->arena.alloc_n<unsigned>(h2g2::N_BAD);
-  pb_h2d(d_us, us, n * 64, s);
-  pb_memset(d_bad, 0xff, h2g2::N_BAD * sizeof(unsigned), s);
-  const int t0 = c->times.begin("h2g2 map", s);
-  pb_launch("h2g2 load u", h2g2::LoadUK{d_us, d_u, d_bad}, n, s, 128);
-  pb_launch("h2g2 map", h2g2::MapK{d_u, d_pts, d_bad}, n, s, 128);
-  pb_launch("h2g2 points", h2g2::PutK{d_pts, d_out, 16}, n, s, 128);
-  c->times.end(t0, s);
-  check_h2g2(c, d_bad);
-  c->times.resolve();
-  pb_d2h(points_out, d_out, n * 128, s);
-  pb_sync(s);
+  on_context(c, n * (8 * 8 + sizeof(h2g2::Fq2) + sizeof(h2g2::Aff) + 16 * 8) + 65536, [&] {
+    const pbStream s = c->stream;
+    u64* d_us = c->arena.alloc_n<u64>(n * 8);
+    h2g2::Fq2* d_u = c->arena.alloc_n<h2g2::Fq2>(n);
+    h2g2::Aff* d_pts = c->arena.alloc_n<h2g2::Aff>(n);
+    u64* d_out = c->arena.alloc_n<u64>(n * 16);
+    unsigned* d_bad = c->arena.alloc_n<unsigned>(h2g2::N_BAD);
+    pb_h2d(d_us, us, n * 64, s);
+    pb_memset(d_bad, 0xff, h2g2::N_BAD * sizeof(unsigned), s);
+    const int t0 = c->times.begin("h2g2 map", s);
+    pb_launch("h2g2 load u", h2g2::LoadUK{d_us, d_u, d_bad}, n, s, 128);
+    pb_launch("h2g2 map", h2g2::MapK{d_u, d_pts, d_bad}, n, s, 128);
+    pb_launch("h2g2 points", h2g2::PutK{d_pts, d_out, 16}, n, s, 128);
+    c->times.end(t0, s);
+    check_h2g2(c, d_bad);
+    pb_d2h(points_out, d_out, n * 128, s);
+  });
 }
 
 void hash_to_g2_impl(pb254_ctx* c, const u64* messages, size_t n, size_t msg_len, u64 seed, u64* inputs_out,
@@ -219,63 +220,61 @@ void hash_to_g2_impl(pb254_ctx* c, const u64* messages, size_t n, size_t msg_len
   using namespace h2g2;
   typedef bn::F2 F;
   const size_t TW = 20, RW = 36, PW = 16;
-  c->arena.reserve(chains::scratch_bytes<F>(n, n) + n * msg_len * 8 +
-                   n * (sizeof(Fq2) + 2 * sizeof(Aff) + 2 * sizeof(Jac) + (TW + 4 + PW + 1 + RW + 2 * PW) * 8) +
-                   65536);
-  c->arena.reset();
-  c->times.clear();
-  const pbStream s = c->stream;
-  if (!c->g2_pow2) {
-    c->g2_pow2 = pb_dev_alloc(TABLE_POINTS * sizeof(Jac));
-    pb_launch("h2g2 table", TableK{(Jac*)c->g2_pow2}, 1, s, 32);
-  }
-  u64* d_msgs = c->arena.alloc_n<u64>(n * msg_len + 1);
-  Fq2* d_u = c->arena.alloc_n<Fq2>(n);
-  Aff* d_pts = c->arena.alloc_n<Aff>(n);
-  u64* d_terms = c->arena.alloc_n<u64>(n * TW);
-  u64* d_k = c->arena.alloc_n<u64>(n * 4);
-  Jac* d_jac = c->arena.alloc_n<Jac>(n);
-  u64* d_offsets = c->arena.alloc_n<u64>(n * PW);
-  u64* d_starts = c->arena.alloc_n<u64>(n + 1);
-  u64* d_rows = c->arena.alloc_n<u64>(n * RW);
-  u64* d_sums = c->arena.alloc_n<u64>(n * PW);
-  u64* d_hashes = c->arena.alloc_n<u64>(n * PW);
-  unsigned* d_bad = c->arena.alloc_n<unsigned>(N_BAD);
-  int* d_err = c->arena.alloc_n<int>(1);  // the affine passes' flag: their points are never at infinity (d_bad)
-  std::vector<u64> starts(n + 1);
-  for (size_t i = 0; i <= n; i++) starts[i] = i;
-  if (msg_len) pb_h2d(d_msgs, messages, n * msg_len * 8, s);
-  pb_h2d(d_starts, starts.data(), (n + 1) * 8, s);
-  pb_memset(d_bad, 0xff, N_BAD * sizeof(unsigned), s);
-  pb_memset(d_err, 0, sizeof(int), s);
+  const size_t bytes = chains::scratch_bytes<F>(n, n) + n * msg_len * 8 +
+                       n * (sizeof(Fq2) + 2 * sizeof(Aff) + 2 * sizeof(Jac) + (TW + 4 + PW + 1 + RW + 2 * PW) * 8) +
+                       65536;
+  on_context(c, bytes, [&] {
+    const pbStream s = c->stream;
+    if (!c->g2_pow2) {
+      c->g2_pow2 = pb_dev_alloc(TABLE_POINTS * sizeof(Jac));
+      pb_launch("h2g2 table", TableK{(Jac*)c->g2_pow2}, 1, s, 32);
+    }
+    u64* d_msgs = c->arena.alloc_n<u64>(n * msg_len + 1);
+    Fq2* d_u = c->arena.alloc_n<Fq2>(n);
+    Aff* d_pts = c->arena.alloc_n<Aff>(n);
+    u64* d_terms = c->arena.alloc_n<u64>(n * TW);
+    u64* d_k = c->arena.alloc_n<u64>(n * 4);
+    Jac* d_jac = c->arena.alloc_n<Jac>(n);
+    u64* d_offsets = c->arena.alloc_n<u64>(n * PW);
+    u64* d_starts = c->arena.alloc_n<u64>(n + 1);
+    u64* d_rows = c->arena.alloc_n<u64>(n * RW);
+    u64* d_sums = c->arena.alloc_n<u64>(n * PW);
+    u64* d_hashes = c->arena.alloc_n<u64>(n * PW);
+    unsigned* d_bad = c->arena.alloc_n<unsigned>(N_BAD);
+    int* d_err = c->arena.alloc_n<int>(1);  // the affine passes' flag: their points are never at infinity (d_bad)
+    std::vector<u64> starts(n + 1);
+    for (size_t i = 0; i <= n; i++) starts[i] = i;
+    if (msg_len) pb_h2d(d_msgs, messages, n * msg_len * 8, s);
+    pb_h2d(d_starts, starts.data(), (n + 1) * 8, s);
+    pb_memset(d_bad, 0xff, N_BAD * sizeof(unsigned), s);
+    pb_memset(d_err, 0, sizeof(int), s);
 
-  int t = c->times.begin("h2g2 hash", s);
-  pb_launch("h2g2 hash", HashK{d_msgs, msg_len, d_u, d_bad}, n, s, 128);
-  c->times.end(t, s);
-  t = c->times.begin("h2g2 map", s);
-  pb_launch("h2g2 map", MapK{d_u, d_pts, d_bad}, n, s, 128);
-  pb_launch("h2g2 terms", CofactorK{d_terms}, n, s, 128);
-  pb_launch("h2g2 points", PutK{d_pts, d_terms + 4, TW}, n, s, 128);
-  c->times.end(t, s);
-  t = c->times.begin("h2g2 offsets", s);
-  pb_launch("h2g2 draw", DrawK{seed, d_k, d_bad}, n, s, 128);
-  fixed_base((const Jac*)c->g2_pow2, d_k, n, d_jac, s);
-  chains::to_affine<F>(d_jac, d_pts, n, d_err, s);
-  pb_launch("h2g2 offsets out", PutK{d_pts, d_offsets, PW}, n, s, 128);
-  c->times.end(t, s);
-  check_h2g2(c, d_bad);
+    int t = c->times.begin("h2g2 hash", s);
+    pb_launch("h2g2 hash", HashK{d_msgs, msg_len, d_u, d_bad}, n, s, 128);
+    c->times.end(t, s);
+    t = c->times.begin("h2g2 map", s);
+    pb_launch("h2g2 map", MapK{d_u, d_pts, d_bad}, n, s, 128);
+    pb_launch("h2g2 terms", CofactorK{d_terms}, n, s, 128);
+    pb_launch("h2g2 points", PutK{d_pts, d_terms + 4, TW}, n, s, 128);
+    c->times.end(t, s);
+    t = c->times.begin("h2g2 offsets", s);
+    pb_launch("h2g2 draw", DrawK{seed, d_k, d_bad}, n, s, 128);
+    fixed_base((const Jac*)c->g2_pow2, d_k, n, d_jac, s);
+    chains::to_affine<F>(d_jac, d_pts, n, d_err, s);
+    pb_launch("h2g2 offsets out", PutK{d_pts, d_offsets, PW}, n, s, 128);
+    c->times.end(t, s);
+    check_h2g2(c, d_bad);
 
-  run_chains<F>(c, d_terms, d_starts, d_offsets, n, starts.data(), n, d_rows, d_sums, inputs_out, nullptr);
+    run_chains<F>(c, d_terms, d_starts, d_offsets, n, starts.data(), n, d_rows, d_sums, inputs_out, nullptr);
 
-  t = c->times.begin("h2g2 outputs", s);
-  pb_launch("h2g2 sub offset", SubOffsetK{d_sums, d_offsets, d_jac, d_bad}, n, s, 128);
-  chains::to_affine<F>(d_jac, d_pts, n, d_err, s);
-  pb_launch("h2g2 hashes out", PutK{d_pts, d_hashes, PW}, n, s, 128);
-  c->times.end(t, s);
-  check_h2g2(c, d_bad);
-  c->times.resolve();
-  pb_d2h(hashes_out, d_hashes, n * PW * 8, s);
-  pb_sync(s);
+    t = c->times.begin("h2g2 outputs", s);
+    pb_launch("h2g2 sub offset", SubOffsetK{d_sums, d_offsets, d_jac, d_bad}, n, s, 128);
+    chains::to_affine<F>(d_jac, d_pts, n, d_err, s);
+    pb_launch("h2g2 hashes out", PutK{d_pts, d_hashes, PW}, n, s, 128);
+    c->times.end(t, s);
+    check_h2g2(c, d_bad);
+    pb_d2h(hashes_out, d_hashes, n * PW * 8, s);
+  });
 }
 
 struct PermuteK {
@@ -288,6 +287,139 @@ struct PermuteK {
     for (int k = 0; k < 12; k++) out[i * 12 + k] = s[k];
   }
 };
+
+// One proof on context c (pb254_prove, _dev, _sharded and _trace). The arena holds the trace words, then either the
+// scratch of `fill` or the prover's workspace. fill(d_trace, results) writes the trace, and the native results where
+// the caller has them, with arena space after the trace that the prover reuses.
+template <class Fill>
+void prove_filled(pb254_ctx* c, int kind, size_t n_rows, const pb254_config& cfg, bool keep_debug,
+                  const pb254_comm* comm, bool trace_is_block, size_t trace_words, size_t fill_bytes, Fill&& fill,
+                  pb254_proof** out) {
+  const size_t workspace = comm ? prover::workspace_bytes_sharded(kind, n_rows, cfg, comm->world)
+                                : prover::workspace_bytes(kind, n_rows, cfg);
+  size_t bytes = trace_words * 8 + std::max(fill_bytes, workspace) + 65536;
+#if !PB_HOSTSIM
+  if (trace_is_block) {  // the estimate is an upper bound: never ask for more than the device has left (the
+                         // collectives of the caller need room too); a proof that really does not fit fails in
+                         // Arena::alloc with PB254_E_OOM
+    const size_t avail = pb_free_bytes(c->device) + c->arena.cap, margin = (size_t)4 << 30;
+    if (avail > margin && bytes > avail - margin) bytes = avail - margin;
+  }
+#endif
+  std::unique_ptr<pb254_proof> pf(new pb254_proof());
+  on_context(c, bytes, [&] {
+    u64* d_trace = c->arena.alloc_n<u64>(trace_words);
+    const size_t mark = c->arena.off;
+    fill(d_trace, pf->results);
+    c->arena.off = mark;
+    prover::prove_device(c, kind, d_trace, n_rows, cfg, pf->data, keep_debug, comm, trace_is_block);
+  });
+  *out = pf.release();
+}
+
+// Whether every rank of a sharded proof can generate only ITS instances: the trace splits into per-rank row blocks of
+// whole instances that each hold the 2^16-row range-check table or none of it (every BASELINE size does). Otherwise
+// (small traces) every rank generates the whole trace.
+bool generate_by_instance(size_t n_rows, size_t world) {
+  return n_rows % world == 0 && (n_rows / world) % tg::PERIOD == 0 && n_rows / world >= 65536;
+}
+
+// generate_trace + prove in one call: what run_once does between src/generators/g1/stark_proof.rs:154 and :163. The
+// trace never leaves the device. comm: one proof across its ranks (include/pb254.h); NULL or world 1 is one GPU.
+int prove_inputs(pb254_ctx* c, int kind, const u64* inputs, const u64* timestamps, size_t n_inputs, size_t min_rows,
+                 const pb254_config* cfg_in, int keep_debug, pb254_proof** out, bool inputs_on_device,
+                 const pb254_comm* comm = nullptr) {
+  return guarded([&] {
+    need(out != nullptr, "null out pointer");
+    need_ctx(c);
+    need_kind(kind);
+    need(inputs && timestamps && n_inputs > 0, "null or empty input");
+    need(!comm || (comm->world && (comm->world & (comm->world - 1)) == 0 && comm->rank < comm->world &&
+                   comm->all_to_all && comm->all_gather),
+         "comm: world must be a power of two, rank < world, callbacks non-null");
+    if (comm && comm->world == 1) comm = nullptr;
+    const tg::Layout l = tg::layout_for(kind);
+    const size_t n_rows = pb254_trace_rows(n_inputs, min_rows);
+    const pb254_config cfg = config_or_default(cfg_in, need_trace_rows(n_rows));
+    if (comm && generate_by_instance(n_rows, comm->world)) {
+      // this rank's row block [rank n / P, (rank + 1) n / P) of the trace, [ceil(W / P) P columns][n / P]
+      const size_t P = comm->world, rk = comm->rank, nloc = n_rows / P;
+      const size_t per = nloc / tg::PERIOD;  // instances per rank
+      const size_t i0 = std::min(n_inputs, rk * per), i1 = std::min(n_inputs, (rk + 1) * per), kloc = i1 - i0;
+      const size_t Wpad = ((size_t)l.width + P - 1) / P * P;
+      const size_t tg_bytes =
+          tg::scratch_bytes(kind, kloc ? kloc : 1) + (kloc + 1) * (l.in_words + 1) * 8 + (P + 1) * 65536 * 8 + 65536;
+      // no native results in this mode: they are spread over the ranks
+      prove_filled(c, kind, n_rows, cfg, keep_debug != 0, comm, true, Wpad * nloc, tg_bytes,
+                   [&](u64* d_rows, std::vector<u64>&) {
+        prover::Stage st(c, "tracegen");
+        u64* d_in = c->arena.alloc_n<u64>(kloc * l.in_words + 1);
+        u64* d_ts = c->arena.alloc_n<u64>(kloc + 1);
+        if (kloc) {
+          pb_h2d(d_in, inputs + i0 * l.in_words, kloc * l.in_words * 8, c->stream);
+          pb_h2d(d_ts, timestamps + i0, kloc * 8, c->stream);
+        }
+        int* d_err = c->arena.alloc_n<int>(1);
+        pb_memset(d_err, 0, sizeof(int), c->stream);
+        tg::generate(c->arena, kind, d_in, d_ts, kloc, nloc, d_rows, d_err, c->stream, rk * nloc);
+        // range-check frequencies: every block counted its own cells into the first 2^16 rows of its frequency
+        // column; the table rows are rows 0 .. 65535 of the whole trace, i.e. of rank 0's block
+        u64* freq = d_rows + (size_t)l.freq * nloc;
+        u64* all = c->arena.alloc_n<u64>(P * 65536);
+        if (comm->all_gather(comm->user, freq, all, 65536 * 8)) throw Pb254Error(PB254_E_CUDA, "collective failed: all_gather");
+        if (rk == 0)
+          pb_launch("sum histograms", prover::SumRecordsK{all, freq, 65536, (int)P}, 65536, c->stream, 128);
+        else
+          pb_memset(freq, 0, 65536 * 8, c->stream);
+        // an input error on one rank must fail the call on every rank (the others would wait in the next collective)
+        u64* e_mine = c->arena.alloc_n<u64>(1);
+        u64* e_all = c->arena.alloc_n<u64>(P);
+        pb_memset(e_mine, 0, 8, c->stream);
+        pb_d2d(e_mine, d_err, sizeof(int), c->stream);
+        if (comm->all_gather(comm->user, e_mine, e_all, 8)) throw Pb254Error(PB254_E_CUDA, "collective failed: all_gather");
+        std::vector<u64> herr(P);
+        pb_d2h(herr.data(), e_all, P * 8, c->stream);
+        pb_sync(c->stream);
+        for (size_t p = 0; p < P; p++) throw_trace_error((int)(herr[p] & 0xffffffffu));
+      }, out);
+    } else {
+      const size_t tg_bytes = tg::scratch_bytes(kind, n_inputs) + n_inputs * (l.in_words + 1) * 8 + 65536;
+      prove_filled(c, kind, n_rows, cfg, keep_debug != 0, comm, false, (size_t)l.width * n_rows, tg_bytes,
+                   [&](u64* d_trace, std::vector<u64>& results) {
+        prover::Stage st(c, "tracegen");
+        const u64 *d_in = inputs, *d_ts = timestamps;
+        if (!inputs_on_device) {
+          u64* hin = c->arena.alloc_n<u64>(n_inputs * l.in_words + 1);
+          u64* hts = c->arena.alloc_n<u64>(n_inputs + 1);
+          pb_h2d(hin, inputs, n_inputs * l.in_words * 8, c->stream);
+          pb_h2d(hts, timestamps, n_inputs * 8, c->stream);
+          d_in = hin;
+          d_ts = hts;
+        }
+        int* d_err = c->arena.alloc_n<int>(1);
+        pb_memset(d_err, 0, sizeof(int), c->stream);
+        tg::generate(c->arena, kind, d_in, d_ts, n_inputs, n_rows, d_trace, d_err, c->stream);
+        int herr = 0;
+        pb_d2h(&herr, d_err, sizeof(int), c->stream);
+        u64* d_res = c->arena.alloc_n<u64>(n_inputs * l.L);
+        pb_launch("gather results", GatherResultsK{d_trace, d_res, n_rows, l.reg1, l.L}, n_inputs * l.L, c->stream,
+                  128);
+        results.resize(n_inputs * l.L);
+        pb_d2h(results.data(), d_res, results.size() * 8, c->stream);
+        pb_sync(c->stream);
+        throw_trace_error(herr);
+      }, out);
+    }
+  });
+}
+
+// the keep_debug artefacts of include/pb254.h; slot 4 and any other slot are empty
+const std::vector<u64>* debug_slot(const pb254_proof* p, int which) {
+  const prover::ProofData& d = p->data;
+  const std::vector<u64>* slots[] = {&d.dbg_aux, &d.dbg_chunks, &d.dbg_challenges, &d.dbg_indices, nullptr,
+                                     &d.dbg_groups};
+  return which >= 0 && which < 6 ? slots[which] : nullptr;
+}
 }  // namespace
 
 extern "C" {
@@ -307,28 +439,29 @@ uint64_t pb254_launch_count(void) { return g_pb_launches.load(); }
 
 int pb254_ctx_create(int device, void* stream, pb254_ctx** out) {
   return guarded([&] {
-    if (!out) throw Pb254Error(PB254_E_BAD_ARG, "null out pointer");
-    PbDeviceGuard device_guard(device);
-    pb254_ctx* c = new pb254_ctx();
+    need(out != nullptr, "null out pointer");
+    std::unique_ptr<pb254_ctx> c(new pb254_ctx());
     c->device = device;
+    // the first call on the new context: no arena yet, and tables.init has drained the stream already
+    on_context(c.get(), 0, [&] {
 #if PB_HOSTSIM
-    c->stream = stream;
+      c->stream = stream;
 #else
-    if (stream) {
-      c->stream = (cudaStream_t)stream;
-    } else {
-      PB_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
-      c->own_stream = true;
-    }
+      if (stream) {
+        c->stream = (cudaStream_t)stream;
+      } else {
+        PB_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
+        c->own_stream = true;
+      }
 #endif
-    c->tables.init(c->stream);
-    *out = c;
+      c->tables.init(c->stream);
+    });
+    *out = c.release();
   });
 }
 
 void pb254_ctx_destroy(pb254_ctx* c) {
   if (!c) return;
-  c->times.clear();
   c->tables.destroy();
   c->arena.destroy();
   if (c->g2_pow2) pb_dev_free(c->g2_pow2);
@@ -347,13 +480,10 @@ double pb254_timing_ms(pb254_ctx* c, int i) {
   return c && i >= 0 && i < (int)c->times.recs.size() ? c->times.recs[i].ms : 0.0;
 }
 
-int pb254_trace_width(int kind) { return kind >= 0 && kind <= 2 ? shape_for(kind).width : -1; }
-int pb254_input_words(int kind) { return kind >= 0 && kind <= 2 ? shape_for(kind).in_words : -1; }
+int pb254_trace_width(int kind) { return valid_kind(kind) ? tg::layout_for(kind).width : -1; }
+int pb254_input_words(int kind) { return valid_kind(kind) ? tg::layout_for(kind).in_words : -1; }
 int pb254_num_aux(int kind, uint32_t nch) {
-  if (kind < 0 || kind > 2) return -1;
-  Shape s = shape_for(kind);
-  int ncols = 3 * s.L + s.aux_len;
-  return ((ncols + 1) / 2 + 1 + 2) * (int)nch;
+  return valid_kind(kind) ? aux::num_aux(tg::layout_for(kind), (int)nch) : -1;
 }
 size_t pb254_trace_rows(size_t n_inputs, size_t min_rows) {
   size_t n = n_inputs * 512 > min_rows ? n_inputs * 512 : min_rows, r = 1;
@@ -364,15 +494,13 @@ size_t pb254_trace_rows(size_t n_inputs, size_t min_rows) {
 int pb254_poseidon_permute(pb254_ctx* c, const uint64_t* in, size_t n, uint64_t* out) {
   return guarded([&] {
     need_ctx(c);
-    PbDeviceGuard device_guard(c->device);
-    c->arena.reserve(2 * n * 96 + 1024);
-    c->arena.reset();
-    u64* din = c->arena.alloc_n<u64>(n * 12);
-    u64* dout = c->arena.alloc_n<u64>(n * 12);
-    pb_h2d(din, in, n * 96, c->stream);
-    pb_launch("poseidon permute", PermuteK{din, dout}, n, c->stream, 128);
-    pb_d2h(out, dout, n * 96, c->stream);
-    pb_sync(c->stream);
+    on_context(c, 2 * n * 96 + 1024, [&] {
+      u64* din = c->arena.alloc_n<u64>(n * 12);
+      u64* dout = c->arena.alloc_n<u64>(n * 12);
+      pb_h2d(din, in, n * 96, c->stream);
+      pb_launch("poseidon permute", PermuteK{din, dout}, n, c->stream, 128);
+      pb_d2h(out, dout, n * 96, c->stream);
+    });
   });
 }
 
@@ -380,19 +508,17 @@ int pb254_lde_batch(pb254_ctx* c, const uint64_t* values, size_t cols, size_t n,
                     uint64_t* lde_out) {
   return guarded([&] {
     need_ctx(c);
-    PbDeviceGuard device_guard(c->device);
     int L = ilog2_strict(n);
     size_t N = n << rate_bits;
-    c->arena.reserve((2 * cols * n + cols * N) * 8 + 4096);
-    c->arena.reset();
-    u64* dv = c->arena.alloc_n<u64>(cols * n);
-    u64* scratch = c->arena.alloc_n<u64>(cols * n);
-    u64* lde = c->arena.alloc_n<u64>(cols * N);
-    pb_h2d(dv, values, cols * n * 8, c->stream);
-    ntt::lde_columns(c->tables, dv, n, lde, N, scratch, (int)cols, L, (int)rate_bits,
-                     from_coeffs ? ntt::FROM_COEFFS_LDE : ntt::FROM_VALUES_LDE, c->stream);
-    pb_d2h(lde_out, lde, cols * N * 8, c->stream);
-    pb_sync(c->stream);
+    on_context(c, (2 * cols * n + cols * N) * 8 + 4096, [&] {
+      u64* dv = c->arena.alloc_n<u64>(cols * n);
+      u64* scratch = c->arena.alloc_n<u64>(cols * n);
+      u64* lde = c->arena.alloc_n<u64>(cols * N);
+      pb_h2d(dv, values, cols * n * 8, c->stream);
+      ntt::lde_columns(c->tables, dv, n, lde, N, scratch, (int)cols, L, (int)rate_bits,
+                       from_coeffs ? ntt::FROM_COEFFS_LDE : ntt::FROM_VALUES_LDE, c->stream);
+      pb_d2h(lde_out, lde, cols * N * 8, c->stream);
+    });
   });
 }
 
@@ -400,31 +526,27 @@ int pb254_commit(pb254_ctx* c, const uint64_t* values, size_t cols, size_t n, ui
                  int from_coeffs, uint64_t* cap_out, uint64_t* digests_out) {
   return guarded([&] {
     need_ctx(c);
-    PbDeviceGuard device_guard(c->device);
     int L = ilog2_strict(n);
     size_t N = n << rate_bits;
     int log_N = L + (int)rate_bits;
     size_t nd = merkle::tree_digests(log_N, (int)cap_height);
-    c->arena.reserve((2 * cols * n + cols * N) * 8 + nd * 32 + 4096);
-    c->arena.reset();
-    u64* dv = c->arena.alloc_n<u64>(cols * n);
-    u64* scratch = c->arena.alloc_n<u64>(cols * n);
-    u64* lde = c->arena.alloc_n<u64>(cols * N);
-    merkle::Digest* dig = c->arena.alloc_n<merkle::Digest>(nd);
-    pb_h2d(dv, values, cols * n * 8, c->stream);
-    c->times.clear();
-    int t0 = c->times.begin("lde", c->stream);
-    ntt::lde_columns(c->tables, dv, n, lde, N, scratch, (int)cols, L, (int)rate_bits,
-                     from_coeffs ? ntt::FROM_COEFFS_LDE : ntt::FROM_VALUES_LDE, c->stream);
-    c->times.end(t0, c->stream);
-    int t1 = c->times.begin("merkle", c->stream);
-    merkle::build_from_lde(lde, N, (int)cols, log_N, (int)cap_height, dig, c->stream);
-    c->times.end(t1, c->stream);
-    size_t ncap = (size_t)1 << cap_height;
-    pb_d2h(cap_out, dig + (nd - ncap), ncap * 32, c->stream);
-    if (digests_out) pb_d2h(digests_out, dig, nd * 32, c->stream);
-    pb_sync(c->stream);
-    c->times.resolve();
+    on_context(c, (2 * cols * n + cols * N) * 8 + nd * 32 + 4096, [&] {
+      u64* dv = c->arena.alloc_n<u64>(cols * n);
+      u64* scratch = c->arena.alloc_n<u64>(cols * n);
+      u64* lde = c->arena.alloc_n<u64>(cols * N);
+      merkle::Digest* dig = c->arena.alloc_n<merkle::Digest>(nd);
+      pb_h2d(dv, values, cols * n * 8, c->stream);
+      int t0 = c->times.begin("lde", c->stream);
+      ntt::lde_columns(c->tables, dv, n, lde, N, scratch, (int)cols, L, (int)rate_bits,
+                       from_coeffs ? ntt::FROM_COEFFS_LDE : ntt::FROM_VALUES_LDE, c->stream);
+      c->times.end(t0, c->stream);
+      int t1 = c->times.begin("merkle", c->stream);
+      merkle::build_from_lde(lde, N, (int)cols, log_N, (int)cap_height, dig, c->stream);
+      c->times.end(t1, c->stream);
+      size_t ncap = (size_t)1 << cap_height;
+      pb_d2h(cap_out, dig + (nd - ncap), ncap * 32, c->stream);
+      if (digests_out) pb_d2h(digests_out, dig, nd * 32, c->stream);
+    });
   });
 }
 
@@ -434,29 +556,25 @@ int pb254_generate_trace(pb254_ctx* c, int kind, const uint64_t* inputs, const u
     need_ctx(c);
     need_kind(kind);
     need(inputs && timestamps && cols_out && n_inputs > 0, "null or empty argument");
-    PbDeviceGuard device_guard(c->device);
     tg::Layout l = tg::layout_for(kind);
     size_t n_rows = pb254_trace_rows(n_inputs, min_rows);
     need_trace_rows(n_rows);
     size_t tbytes = (size_t)l.width * n_rows * 8;
-    c->arena.reserve(tbytes + tg::scratch_bytes(kind, n_inputs) + n_inputs * (l.in_words + 1) * 8 + 65536);
-    c->arena.reset();
-    u64* d_trace = c->arena.alloc_n<u64>((size_t)l.width * n_rows);
-    u64* d_in = c->arena.alloc_n<u64>(n_inputs * l.in_words + 1);
-    u64* d_ts = c->arena.alloc_n<u64>(n_inputs + 1);
-    int* d_err = c->arena.alloc_n<int>(1);
-    pb_h2d(d_in, inputs, n_inputs * l.in_words * 8, c->stream);
-    pb_h2d(d_ts, timestamps, n_inputs * 8, c->stream);
-    pb_memset(d_err, 0, sizeof(int), c->stream);
-    c->times.clear();
-    int t0 = c->times.begin("tracegen", c->stream);
-    tg::generate(c->arena, kind, d_in, d_ts, n_inputs, n_rows, d_trace, d_err, c->stream);
-    c->times.end(t0, c->stream);
     int herr = 0;
-    pb_d2h(&herr, d_err, sizeof(int), c->stream);
-    pb_d2h(cols_out, d_trace, tbytes, c->stream);
-    pb_sync(c->stream);
-    c->times.resolve();
+    on_context(c, tbytes + tg::scratch_bytes(kind, n_inputs) + n_inputs * (l.in_words + 1) * 8 + 65536, [&] {
+      u64* d_trace = c->arena.alloc_n<u64>((size_t)l.width * n_rows);
+      u64* d_in = c->arena.alloc_n<u64>(n_inputs * l.in_words + 1);
+      u64* d_ts = c->arena.alloc_n<u64>(n_inputs + 1);
+      int* d_err = c->arena.alloc_n<int>(1);
+      pb_h2d(d_in, inputs, n_inputs * l.in_words * 8, c->stream);
+      pb_h2d(d_ts, timestamps, n_inputs * 8, c->stream);
+      pb_memset(d_err, 0, sizeof(int), c->stream);
+      int t0 = c->times.begin("tracegen", c->stream);
+      tg::generate(c->arena, kind, d_in, d_ts, n_inputs, n_rows, d_trace, d_err, c->stream);
+      c->times.end(t0, c->stream);
+      pb_d2h(&herr, d_err, sizeof(int), c->stream);
+      pb_d2h(cols_out, d_trace, tbytes, c->stream);
+    });
     throw_trace_error(herr);
   });
 }
@@ -475,7 +593,6 @@ int pb254_scalar_mul_chains(pb254_ctx* c, int kind, const uint64_t* terms, size_
          "chain_starts must begin at 0 and end at n_terms");
     for (size_t k = 0; k < n_chains; k++) need(chain_starts[k] <= chain_starts[k + 1], "chain_starts must not decrease");
     if (n_chains == 0) return;
-    PbDeviceGuard device_guard(c->device);
     if (kind == PB254_KIND_G1)
       scalar_mul_chains_impl<bn::F1>(c, terms, n_terms, chain_starts, n_chains, offsets, inputs_out, sums_out);
     else
@@ -489,7 +606,6 @@ int pb254_map_to_g2(pb254_ctx* c, const uint64_t* us, size_t n, uint64_t* points
     need(n <= h2g2::MAX_N, "more than 2^17 values");
     if (n == 0) return;
     need(us && points_out, "null us or points_out");
-    PbDeviceGuard device_guard(c->device);
     map_to_g2_impl(c, us, n, points_out);
   });
 }
@@ -502,169 +618,18 @@ int pb254_hash_to_g2(pb254_ctx* c, const uint64_t* messages, size_t n, size_t ms
     need(msg_len <= h2g2::MAX_MSG_ELEMS && n * msg_len <= h2g2::MAX_MSG_ELEMS, "more than 2^24 message elements");
     if (n == 0) return;
     need((messages || msg_len == 0) && inputs_out && hashes_out, "null messages, inputs_out or hashes_out");
-    PbDeviceGuard device_guard(c->device);
     hash_to_g2_impl(c, messages, n, msg_len, seed, inputs_out, hashes_out);
   });
 }
 
-// generate_trace + prove in one call: what run_once does between
-// src/generators/g1/stark_proof.rs:154 and :163. The trace never leaves the device.
-static int prove_inputs_impl(pb254_ctx* c, int kind, const uint64_t* inputs, const uint64_t* timestamps, size_t n_inputs,
-                             size_t min_rows, const pb254_config* cfg_in, int keep_debug, pb254_proof** out,
-                             bool inputs_on_device, const pb254_comm* comm = nullptr) {
-  return guarded([&] {
-    need(out != nullptr, "null out pointer");
-    need_ctx(c);
-    need_kind(kind);
-    need(inputs && timestamps && n_inputs > 0, "null or empty input");
-    PbDeviceGuard device_guard(c->device);
-    tg::Layout l = tg::layout_for(kind);
-    size_t n_rows = pb254_trace_rows(n_inputs, min_rows);
-    const pb254_config cfg = config_or_default(cfg_in, need_trace_rows(n_rows));
-    size_t twords = (size_t)l.width * n_rows;
-    size_t tg_bytes = tg::scratch_bytes(kind, n_inputs) + n_inputs * (l.in_words + 1) * 8 + 65536;
-    need(!comm || (comm->world >= 1 && (comm->world & (comm->world - 1)) == 0 && comm->rank < comm->world),
-         "comm: world must be a power of two and rank < world");
-    size_t pv_bytes = comm && comm->world > 1 ? prover::workspace_bytes_sharded(kind, n_rows, cfg, comm->world)
-                                              : prover::workspace_bytes(kind, n_rows, cfg);
-    c->arena.reserve(twords * 8 + (tg_bytes > pv_bytes ? tg_bytes : pv_bytes) + 65536);
-    c->arena.reset();
-    c->times.clear();
-    u64* d_trace = c->arena.alloc_n<u64>(twords);
-    size_t mark = c->arena.off;
-    std::vector<u64> results;
-    {
-      prover::Stage st(c, "tracegen");
-      const u64 *d_in = inputs, *d_ts = timestamps;
-      if (!inputs_on_device) {
-        u64* hin = c->arena.alloc_n<u64>(n_inputs * l.in_words + 1);
-        u64* hts = c->arena.alloc_n<u64>(n_inputs + 1);
-        pb_h2d(hin, inputs, n_inputs * l.in_words * 8, c->stream);
-        pb_h2d(hts, timestamps, n_inputs * 8, c->stream);
-        d_in = hin;
-        d_ts = hts;
-      }
-      int* d_err = c->arena.alloc_n<int>(1);
-      pb_memset(d_err, 0, sizeof(int), c->stream);
-      tg::generate(c->arena, kind, d_in, d_ts, n_inputs, n_rows, d_trace, d_err, c->stream);
-      int herr = 0;
-      pb_d2h(&herr, d_err, sizeof(int), c->stream);
-      u64* d_res = c->arena.alloc_n<u64>(n_inputs * l.L);
-      pb_launch("gather results", GatherResultsK{d_trace, d_res, n_rows, l.reg1, l.L}, n_inputs * l.L, c->stream, 128);
-      results.resize(n_inputs * l.L);
-      pb_d2h(results.data(), d_res, results.size() * 8, c->stream);
-      pb_sync(c->stream);
-      throw_trace_error(herr);
-    }
-    c->arena.off = mark;
-    pb254_proof* pf = new pb254_proof();
-    pf->results.swap(results);
-    try {
-      prover::prove_device(c, kind, d_trace, n_rows, cfg, pf->data, keep_debug != 0, comm);
-    } catch (...) {
-      delete pf;
-      throw;
-    }
-    pb_sync(c->stream);
-    c->times.resolve();
-    *out = pf;
-  });
-}
-
-// One proof across the ranks of `comm` (include/pb254.h). When the trace splits into per-rank row blocks of whole
-// instances that each hold the 2^16-row range-check table or none of it (n / world a multiple of 512 and >= 65536 -
-// every BASELINE size does), every rank generates only ITS instances: the row block [rank n / P, (rank + 1) n / P) of
-// the trace; the range-check histogram is added up across the ranks and lands in rank 0's frequency column. Otherwise
-// (small traces) every rank generates the whole trace. world == 1 (or comm == NULL) is pb254_prove.
 int pb254_prove_sharded(pb254_ctx* c, int kind, const uint64_t* inputs, const uint64_t* timestamps, size_t n_inputs,
                         size_t min_rows, const pb254_config* cfg_in, const pb254_comm* comm, pb254_proof** out) {
-  if (!comm || comm->world <= 1)
-    return prove_inputs_impl(c, kind, inputs, timestamps, n_inputs, min_rows, cfg_in, 0, out, false, comm);
-  {
-    const size_t n_rows = pb254_trace_rows(n_inputs, min_rows), P = comm->world;
-    const bool pow2 = P && (P & (P - 1)) == 0;
-    if (!pow2 || n_rows % P || (n_rows / P) % tg::PERIOD || n_rows / P < 65536)
-      return prove_inputs_impl(c, kind, inputs, timestamps, n_inputs, min_rows, cfg_in, 0, out, false, comm);
-  }
-  return guarded([&] {
-    need(out != nullptr, "null out pointer");
-    need_ctx(c);
-    need_kind(kind);
-    need(inputs && timestamps && n_inputs > 0, "null or empty input");
-    need(comm->rank < comm->world && comm->all_to_all && comm->all_gather, "comm: rank < world, callbacks non-null");
-    PbDeviceGuard device_guard(c->device);
-    const tg::Layout l = tg::layout_for(kind);
-    const size_t n_rows = pb254_trace_rows(n_inputs, min_rows), P = comm->world, rk = comm->rank, nloc = n_rows / P;
-    const pb254_config cfg = config_or_default(cfg_in, need_trace_rows(n_rows));
-    const size_t per = nloc / tg::PERIOD;  // instances per rank
-    const size_t i0 = std::min(n_inputs, rk * per), i1 = std::min(n_inputs, (rk + 1) * per), kloc = i1 - i0;
-    const size_t Wpad = ((size_t)l.width + P - 1) / P * P;
-    const size_t twords = Wpad * nloc;
-    size_t tg_bytes = tg::scratch_bytes(kind, kloc ? kloc : 1) + (kloc + 1) * (l.in_words + 1) * 8 + (P + 1) * 65536 * 8 + 65536;
-    size_t pv_bytes = prover::workspace_bytes_sharded(kind, n_rows, cfg, P);
-    size_t want = twords * 8 + (tg_bytes > pv_bytes ? tg_bytes : pv_bytes) + 65536;
-#if !PB_HOSTSIM
-    {  // the estimate is an upper bound: never ask for more than the device has left (the collectives of the caller
-       // need room too); a proof that really does not fit fails in Arena::alloc with PB254_E_OOM
-      size_t free_b = 0, total_b = 0;
-      PB_CUDA(cudaMemGetInfo(&free_b, &total_b));
-      const size_t avail = free_b + c->arena.cap, margin = (size_t)4 << 30;
-      if (avail > margin && want > avail - margin) want = avail - margin;
-    }
-#endif
-    c->arena.reserve(want);
-    c->arena.reset();
-    c->times.clear();
-    u64* d_rows = c->arena.alloc_n<u64>(twords);
-    size_t mark = c->arena.off;
-    {
-      prover::Stage st(c, "tracegen");
-      u64* d_in = c->arena.alloc_n<u64>(kloc * l.in_words + 1);
-      u64* d_ts = c->arena.alloc_n<u64>(kloc + 1);
-      if (kloc) {
-        pb_h2d(d_in, inputs + i0 * l.in_words, kloc * l.in_words * 8, c->stream);
-        pb_h2d(d_ts, timestamps + i0, kloc * 8, c->stream);
-      }
-      int* d_err = c->arena.alloc_n<int>(1);
-      pb_memset(d_err, 0, sizeof(int), c->stream);
-      tg::generate(c->arena, kind, d_in, d_ts, kloc, nloc, d_rows, d_err, c->stream, rk * nloc);
-      // range-check frequencies: every block counted its own cells into the first 2^16 rows of its frequency column;
-      // the table rows are rows 0 .. 65535 of the whole trace, i.e. of rank 0's block
-      u64* freq = d_rows + (size_t)l.freq * nloc;
-      u64* all = c->arena.alloc_n<u64>(P * 65536);
-      if (comm->all_gather(comm->user, freq, all, 65536 * 8)) throw Pb254Error(PB254_E_CUDA, "collective failed: all_gather");
-      if (rk == 0)
-        pb_launch("sum histograms", prover::SumRecordsK{all, freq, 65536, (int)P}, 65536, c->stream, 128);
-      else
-        pb_memset(freq, 0, 65536 * 8, c->stream);
-      // an input error on one rank must fail the call on every rank (the others would wait in the next collective)
-      u64* e_mine = c->arena.alloc_n<u64>(1);
-      u64* e_all = c->arena.alloc_n<u64>(P);
-      pb_memset(e_mine, 0, 8, c->stream);
-      pb_d2d(e_mine, d_err, sizeof(int), c->stream);
-      if (comm->all_gather(comm->user, e_mine, e_all, 8)) throw Pb254Error(PB254_E_CUDA, "collective failed: all_gather");
-      std::vector<u64> herr(P);
-      pb_d2h(herr.data(), e_all, P * 8, c->stream);
-      pb_sync(c->stream);
-      for (size_t p = 0; p < P; p++) throw_trace_error((int)(herr[p] & 0xffffffffu));
-    }
-    c->arena.off = mark;
-    pb254_proof* pf = new pb254_proof();  // no native results in this mode: they are spread over the ranks
-    try {
-      prover::prove_device(c, kind, d_rows, n_rows, cfg, pf->data, false, comm, true);
-    } catch (...) {
-      delete pf;
-      throw;
-    }
-    pb_sync(c->stream);
-    c->times.resolve();
-    *out = pf;
-  });
+  return prove_inputs(c, kind, inputs, timestamps, n_inputs, min_rows, cfg_in, 0, out, false, comm);
 }
 
 int pb254_prove(pb254_ctx* c, int kind, const uint64_t* inputs, const uint64_t* timestamps, size_t n_inputs,
                 size_t min_rows, const pb254_config* cfg, int keep_debug, pb254_proof** out) {
-  return prove_inputs_impl(c, kind, inputs, timestamps, n_inputs, min_rows, cfg, keep_debug, out, false);
+  return prove_inputs(c, kind, inputs, timestamps, n_inputs, min_rows, cfg, keep_debug, out, false);
 }
 
 int pb254_prove_many(pb254_ctx* const* ctxs, size_t n_ctx, int kind, const uint64_t* inputs, const uint64_t* timestamps,
@@ -679,7 +644,7 @@ int pb254_prove_many(pb254_ctx* const* ctxs, size_t n_ctx, int kind, const uint6
     }
   });
   if (rc) return rc;
-  const size_t in_words = (size_t)shape_for(kind).in_words;
+  const size_t in_words = (size_t)tg::layout_for(kind).in_words;
   for (size_t b = 0; b < n_batches; b++) proofs_out[b] = nullptr;
   std::vector<int> codes(n_ctx, 0);
   std::vector<std::string> messages(n_ctx);
@@ -708,7 +673,7 @@ int pb254_prove_many(pb254_ctx* const* ctxs, size_t n_ctx, int kind, const uint6
 // Same with `inputs` / `timestamps` already resident in device memory of the context's GPU.
 int pb254_prove_dev(pb254_ctx* c, int kind, const uint64_t* d_inputs, const uint64_t* d_timestamps, size_t n_inputs,
                     size_t min_rows, const pb254_config* cfg, int keep_debug, pb254_proof** out) {
-  return prove_inputs_impl(c, kind, d_inputs, d_timestamps, n_inputs, min_rows, cfg, keep_debug, out, true);
+  return prove_inputs(c, kind, d_inputs, d_timestamps, n_inputs, min_rows, cfg, keep_debug, out, true);
 }
 
 // prove(stark, config, trace, ...) on a host trace (column-major width x n_rows), the literal
@@ -720,19 +685,14 @@ int pb254_prove_trace(pb254_ctx* c, int kind, const uint64_t* trace_cols, size_t
     need_ctx(c);
     need_kind(kind);
     need(trace_cols != nullptr, "null trace");
-    PbDeviceGuard device_guard(c->device);
     const pb254_config cfg = config_or_default(cfg_in, need_trace_rows(n_rows));
-    tg::Layout l = tg::layout_for(kind);
-    size_t twords = (size_t)l.width * n_rows;
-    c->arena.reserve(twords * 8 + prover::workspace_bytes(kind, n_rows, cfg) + 65536);
-    c->arena.reset();
-    c->times.clear();
-    u64* d_trace = c->arena.alloc_n<u64>(twords);
-    pb_h2d(d_trace, trace_cols, twords * 8, c->stream);
-    {
+    const tg::Layout l = tg::layout_for(kind);
+    const size_t twords = (size_t)l.width * n_rows;
+    prove_filled(c, kind, n_rows, cfg, keep_debug != 0, nullptr, false, twords, 0,
+                 [&](u64* d_trace, std::vector<u64>&) {
+      pb_h2d(d_trace, trace_cols, twords * 8, c->stream);
       // A host-supplied trace has not been through generate_range_checks: every looked-up cell and the table column
       // must be < 2^16 (the reference asserts this while filling the frequency column, g1/scalar_mul_stark.rs:71-87).
-      size_t mark = c->arena.off;
       int* d_err = c->arena.alloc_n<int>(1);
       pb_memset(d_err, 0, sizeof(int), c->stream);
       pb_launch("range pre-check", aux::RangePrecheckK{d_trace, n_rows, l.rc_lo, l.rc_hi, l.range_counter, d_err},
@@ -740,19 +700,8 @@ int pb254_prove_trace(pb254_ctx* c, int kind, const uint64_t* trace_cols, size_t
       int herr = 0;
       pb_d2h(&herr, d_err, sizeof(int), c->stream);
       pb_sync(c->stream);
-      c->arena.off = mark;
       if (herr) throw Pb254Error(PB254_E_BAD_ARG, "trace: a range-checked cell or the range counter is >= 2^16");
-    }
-    pb254_proof* pf = new pb254_proof();
-    try {
-      prover::prove_device(c, kind, d_trace, n_rows, cfg, pf->data, keep_debug != 0);
-    } catch (...) {
-      delete pf;
-      throw;
-    }
-    pb_sync(c->stream);
-    c->times.resolve();
-    *out = pf;
+    }, out);
   });
 }
 
@@ -762,18 +711,14 @@ int pb254_lde_dev(pb254_ctx* c, const uint64_t* d_values, size_t cols, size_t n,
                   uint64_t* d_lde_out) {
   return guarded([&] {
     need_ctx(c);
-    PbDeviceGuard device_guard(c->device);
     int L = ilog2_strict(n);
-    c->arena.reserve(cols * n * 8 + 4096);
-    c->arena.reset();
-    u64* scratch = c->arena.alloc_n<u64>(cols * n);
-    c->times.clear();
-    int t0 = c->times.begin("lde", c->stream);
-    ntt::lde_columns(c->tables, d_values, n, d_lde_out, n << rate_bits, scratch, (int)cols, L, (int)rate_bits,
-                     from_coeffs ? ntt::FROM_COEFFS_LDE : ntt::FROM_VALUES_LDE, c->stream);
-    c->times.end(t0, c->stream);
-    pb_sync(c->stream);
-    c->times.resolve();
+    on_context(c, cols * n * 8 + 4096, [&] {
+      u64* scratch = c->arena.alloc_n<u64>(cols * n);
+      int t0 = c->times.begin("lde", c->stream);
+      ntt::lde_columns(c->tables, d_values, n, d_lde_out, n << rate_bits, scratch, (int)cols, L, (int)rate_bits,
+                       from_coeffs ? ntt::FROM_COEFFS_LDE : ntt::FROM_VALUES_LDE, c->stream);
+      c->times.end(t0, c->stream);
+    });
   });
 }
 
@@ -781,13 +726,11 @@ int pb254_leaf_hash_rows_dev(pb254_ctx* c, const uint64_t* d_matrix, size_t stri
                              uint64_t* d_digests_out) {
   return guarded([&] {
     need_ctx(c);
-    PbDeviceGuard device_guard(c->device);
-    c->times.clear();
-    int t0 = c->times.begin("leaf hash rows", c->stream);
-    merkle::hash_rows_natural(d_matrix, stride, (int)cols, rows, (merkle::Digest*)d_digests_out, c->stream);
-    c->times.end(t0, c->stream);
-    pb_sync(c->stream);
-    c->times.resolve();
+    on_context(c, 0, [&] {
+      int t0 = c->times.begin("leaf hash rows", c->stream);
+      merkle::hash_rows_natural(d_matrix, stride, (int)cols, rows, (merkle::Digest*)d_digests_out, c->stream);
+      c->times.end(t0, c->stream);
+    });
   });
 }
 
@@ -797,22 +740,18 @@ int pb254_merkle_subtree_dev(pb254_ctx* c, const uint64_t* d_all_digests, uint32
                              uint32_t log_sub, uint32_t log_roots, uint64_t* d_roots_out) {
   return guarded([&] {
     need_ctx(c);
-    PbDeviceGuard device_guard(c->device);
     if (log_roots > log_sub || log_sub > log_total) throw Pb254Error(PB254_E_BAD_ARG, "subtree shape");
     size_t nd = merkle::tree_digests((int)log_sub, (int)log_roots);
-    c->arena.reserve(nd * 32 + 4096);
-    c->arena.reset();
-    merkle::Digest* dig = c->arena.alloc_n<merkle::Digest>(nd);
-    c->times.clear();
-    int t0 = c->times.begin("subtree", c->stream);
-    pb_launch("subtree leaves", merkle::SubtreeLeavesK{(const merkle::Digest*)d_all_digests, dig, first, (int)log_total},
-              (size_t)1 << log_sub, c->stream, 128);
-    merkle::build_levels(dig, (int)log_sub, (int)log_roots, c->stream);
-    size_t nr = (size_t)1 << log_roots;
-    pb_d2d(d_roots_out, dig + (nd - nr), nr * 32, c->stream);
-    c->times.end(t0, c->stream);
-    pb_sync(c->stream);
-    c->times.resolve();
+    on_context(c, nd * 32 + 4096, [&] {
+      merkle::Digest* dig = c->arena.alloc_n<merkle::Digest>(nd);
+      int t0 = c->times.begin("subtree", c->stream);
+      pb_launch("subtree leaves", merkle::SubtreeLeavesK{(const merkle::Digest*)d_all_digests, dig, first, (int)log_total},
+                (size_t)1 << log_sub, c->stream, 128);
+      merkle::build_levels(dig, (int)log_sub, (int)log_roots, c->stream);
+      size_t nr = (size_t)1 << log_roots;
+      pb_d2d(d_roots_out, dig + (nd - nr), nr * 32, c->stream);
+      c->times.end(t0, c->stream);
+    });
   });
 }
 
@@ -837,9 +776,12 @@ int pb254_verify_device(pb254_ctx* c, int kind, const pb254_config* cfg_in, cons
     need_kind(kind);
     need(proof_words && inputs && timestamps, "null argument");
     const pb254_config cfg = config_or_default(cfg_in, -1);
-    PbDeviceGuard device_guard(c->device);
-    verify_dev::DeviceChecks checks(c);
-    verify::verify_walk(kind, cfg, proof_words, n_words, inputs, timestamps, n_inputs, checks);
+    on_context(c, 0, [&] {
+      // DeviceChecks sizes the arena once the walk knows the proof's shape, and its destructor drains the stream on
+      // every path (a walk that fails early leaves kernels in flight); the scope's own drain then finds it empty
+      verify_dev::DeviceChecks checks(c);
+      verify::verify_walk(kind, cfg, proof_words, n_words, inputs, timestamps, n_inputs, checks);
+    });
   });
 }
 
@@ -855,16 +797,12 @@ int pb254_proof_parse(const uint64_t* proof_words, size_t n_words, pb254_proof_l
 
 size_t pb254_proof_words(const pb254_proof* p) { return p->data.blob.size(); }
 const uint64_t* pb254_proof_data(const pb254_proof* p) { return p->data.blob.data(); }
-// debug artefacts kept when keep_debug != 0: 0 auxiliary values (A x n), 1 quotient chunk coefficients
-// (2*num_challenges x n), 2 challenges [betas, gammas, alphas, zeta, fri_alpha, fri_betas], 3 query indices
 size_t pb254_proof_debug_words(const pb254_proof* p, int which) {
-  const std::vector<u64>* v = which == 0 ? &p->data.dbg_aux : which == 1 ? &p->data.dbg_chunks
-                            : which == 2 ? &p->data.dbg_challenges : which == 3 ? &p->data.dbg_indices : which == 4 ? &p->data.dbg_qvals : which == 5 ? &p->data.dbg_groups : nullptr;
+  const std::vector<u64>* v = debug_slot(p, which);
   return v ? v->size() : 0;
 }
 const uint64_t* pb254_proof_debug_data(const pb254_proof* p, int which) {
-  const std::vector<u64>* v = which == 0 ? &p->data.dbg_aux : which == 1 ? &p->data.dbg_chunks
-                            : which == 2 ? &p->data.dbg_challenges : which == 3 ? &p->data.dbg_indices : which == 4 ? &p->data.dbg_qvals : which == 5 ? &p->data.dbg_groups : nullptr;
+  const std::vector<u64>* v = debug_slot(p, which);
   return v ? v->data() : nullptr;
 }
 

@@ -65,7 +65,7 @@ static const u64 PROOF_MAGIC = proofview::MAGIC;
 
 struct ProofData {
   std::vector<u64> blob;
-  std::vector<u64> dbg_aux, dbg_chunks, dbg_challenges, dbg_indices, dbg_qvals, dbg_groups;
+  std::vector<u64> dbg_aux, dbg_chunks, dbg_challenges, dbg_indices, dbg_groups;
 };
 
 static inline void validate_config(const pb254_config& c) {
@@ -163,11 +163,8 @@ static inline void prove_device(pb254_ctx* c, int kind, const u64* d_trace, size
   const bool sharded = comm && comm->world > 1;
   const size_t P = sharded ? comm->world : 1, rk = sharded ? comm->rank : 0;
   const size_t Nloc = N / P, halo = (size_t)1 << r;  // LDE rows per rank; the next trace row is 2^r LDE rows further
-  if (sharded) {
-    if ((P & (P - 1)) || rk >= P || !comm->all_to_all || !comm->all_gather)
-      throw Pb254Error(PB254_E_BAD_ARG, "comm: world must be a power of two, rank < world, callbacks non-null");
-    if (Nloc < 256 || keep_debug) throw Pb254Error(PB254_E_BAD_ARG, "comm: too many ranks for this trace (or keep_debug set)");
-  }
+  if (sharded && (Nloc < 256 || keep_debug))
+    throw Pb254Error(PB254_E_BAD_ARG, "comm: too many ranks for this trace (or keep_debug set)");
   auto coll = [&](int rc, const char* what) {
     if (rc) throw Pb254Error(PB254_E_CUDA, std::string("collective failed: ") + what);
   };
@@ -787,8 +784,6 @@ static inline void prove_device(pb254_ctx* c, int kind, const u64* d_trace, size
     pb_d2h(out.dbg_aux.data(), aux_vals, (size_t)A * n * 8, s);
     out.dbg_chunks.resize((size_t)Q * n);
     pb_d2h(out.dbg_chunks.data(), qcoef, (size_t)Q * n * 8, s);
-    out.dbg_qvals.resize((size_t)nch * qsize);
-    pb_d2h(out.dbg_qvals.data(), qvals, (size_t)nch * qsize * 8, s);
     out.dbg_groups.resize(4096);
     pb_d2h(out.dbg_groups.data(), d_dbg_groups, 4096 * 8, s);
     pb_sync(s);

@@ -124,7 +124,7 @@ struct DeviceChecks : verify::Checks {
   u64* d_sum = nullptr;
   std::vector<int> ok;
   bool have_ok = false;
-  explicit DeviceChecks(pb254_ctx* ctx) : c(ctx) { c->times.clear(); }
+  explicit DeviceChecks(pb254_ctx* ctx) : c(ctx) {}
   ~DeviceChecks() override {
 #if !PB_HOSTSIM
     (void)cudaStreamSynchronize(c->stream);  // errors of the stream are reported by the next call on the context
