@@ -218,6 +218,20 @@ int pb254_verify(int kind, const pb254_config* cfg, const uint64_t* proof_words,
  * "verify merkle" (pb254_timing_*). */
 int pb254_verify_device(pb254_ctx* ctx, int kind, const pb254_config* cfg, const uint64_t* proof_words,
                         size_t n_words, const uint64_t* inputs, const uint64_t* timestamps, size_t n_inputs);
+#define PB254_VERIFY_MESSAGE_BYTES 256
+/* pb254_verify_device on n_proofs proofs of ONE kind under ONE StarkConfig (the caller's, NULL = standard_fast), the
+ * batched counterpart of pb254_prove_many: one launch per stage for every 64 proofs.
+ * proof_words[b] / n_words[b]: proof b. inputs / timestamps: the batches of all proofs concatenated in the pb254_prove
+ * wire format; proof b's rows are input_starts[b] .. input_starts[b+1] (n_proofs + 1 indices, input_starts[0] = 0,
+ * non-decreasing). codes_out[b]: what pb254_verify returns for proof b alone (0 = accepted). messages_out: NULL, or
+ * n_proofs slots of PB254_VERIFY_MESSAGE_BYTES; slot b receives pb254_last_error() of that pb254_verify call,
+ * NUL-terminated and truncated to fit ("" for an accepted proof).
+ * Returns PB254_OK if every proof is accepted. Otherwise it returns the code of the lowest rejected proof, and
+ * pb254_last_error() is "proof <b>: <its message>". PB254_E_CUDA / PB254_E_OOM fail the whole call and are written
+ * to every codes_out entry. PB254_E_BAD_ARG for bad arguments leaves the outputs untouched. At most 2^12 proofs. */
+int pb254_verify_many_device(pb254_ctx* ctx, int kind, const pb254_config* cfg, const uint64_t* const* proof_words,
+                             const size_t* n_words, size_t n_proofs, const uint64_t* inputs, const uint64_t* timestamps,
+                             const uint64_t* input_starts, int* codes_out, char* messages_out);
 /* Serialized StarkProofWithMetadata: little-endian u64 words, field order of SURVEY.md C.7 behind a
  * 10-word header {magic, kind, degree_bits, config[7]} (layout in DESIGN.md). */
 size_t pb254_proof_words(const pb254_proof* proof);

@@ -776,13 +776,59 @@ int pb254_verify_device(pb254_ctx* c, int kind, const pb254_config* cfg_in, cons
     need_kind(kind);
     need(proof_words && inputs && timestamps, "null argument");
     const pb254_config cfg = config_or_default(cfg_in, -1);
+    const uint64_t starts[2] = {0, n_inputs};
+    verify_dev::Outcome o;
+    // the batch of one: the round's coordinator sizes the arena once the walk knows the proof's shape, and drains the
+    // stream before the walk reads its results
     on_context(c, 0, [&] {
-      // DeviceChecks sizes the arena once the walk knows the proof's shape, and its destructor drains the stream on
-      // every path (a walk that fails early leaves kernels in flight); the scope's own drain then finds it empty
-      verify_dev::DeviceChecks checks(c);
-      verify::verify_walk(kind, cfg, proof_words, n_words, inputs, timestamps, n_inputs, checks);
+      verify_dev::verify_many(c, kind, cfg, &proof_words, &n_words, 1, inputs, timestamps, starts, &o);
     });
+    if (o.code) throw Pb254Error(o.code, o.msg);
   });
+}
+
+// pb254_verify_device on n_proofs proofs in rounds of verify_dev::ROUND: one launch per stage per round.
+int pb254_verify_many_device(pb254_ctx* c, int kind, const pb254_config* cfg_in, const uint64_t* const* proof_words,
+                             const size_t* n_words, size_t n_proofs, const uint64_t* inputs, const uint64_t* timestamps,
+                             const uint64_t* input_starts, int* codes_out, char* messages_out) {
+  std::vector<verify_dev::Outcome> out;
+  const int rc = guarded([&] {
+    need_ctx(c);
+    need_kind(kind);
+    need(n_proofs <= verify_dev::MAX_PROOFS, "more than 2^12 proofs");
+    need(proof_words && n_words && inputs && timestamps && input_starts && codes_out, "null argument");
+    for (size_t b = 0; b < n_proofs; b++) need(proof_words[b] != nullptr, "null proof_words entry");
+    need(input_starts[0] == 0, "input_starts[0] must be 0");
+    for (size_t b = 0; b < n_proofs; b++) need(input_starts[b] <= input_starts[b + 1], "input_starts must not decrease");
+    const pb254_config cfg = config_or_default(cfg_in, -1);
+    out.resize(n_proofs);
+    try {
+      on_context(c, 0, [&] {
+        verify_dev::verify_many(c, kind, cfg, proof_words, n_words, n_proofs, inputs, timestamps, input_starts,
+                                out.data());
+      });
+    } catch (const Pb254Error& e) {  // PB254_E_CUDA / PB254_E_OOM fail every proof
+      for (auto& o : out) o = verify_dev::Outcome{e.code, e.what()};
+      throw;
+    }
+  });
+  if (out.empty()) return rc;  // bad arguments (outputs untouched), or no proofs
+  for (size_t b = 0; b < n_proofs; b++) {
+    codes_out[b] = out[b].code;
+    if (messages_out) {
+      char* m = messages_out + b * PB254_VERIFY_MESSAGE_BYTES;
+      const size_t len = std::min(out[b].msg.size(), (size_t)PB254_VERIFY_MESSAGE_BYTES - 1);
+      memcpy(m, out[b].msg.data(), len);
+      m[len] = 0;
+    }
+  }
+  if (rc) return rc;
+  for (size_t b = 0; b < n_proofs; b++)
+    if (out[b].code) {
+      g_last_error = "proof " + std::to_string(b) + ": " + out[b].msg;
+      return out[b].code;
+    }
+  return PB254_OK;
 }
 
 void pb254_proof_free(pb254_proof* p) { delete p; }

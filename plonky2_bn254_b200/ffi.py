@@ -15,6 +15,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libpb254.so")
 
 KIND_G1, KIND_G2, KIND_FQ = 0, 1, 2
+MESSAGE_BYTES = 256  # PB254_VERIFY_MESSAGE_BYTES
 
 ERROR_NAMES = {
     0: "OK", 1: "E_SCALAR_RANGE", 2: "E_INFINITY", 3: "E_NOT_CANONICAL", 4: "E_CUDA", 5: "E_OOM", 6: "E_BAD_ARG",
@@ -107,6 +108,10 @@ class Library:
         L.pb254_proof_results_data.argtypes = [C.c_void_p]
 
         L.pb254_proof_parse.argtypes = [C.c_void_p, C.c_size_t, C.POINTER(ProofLayout)]
+        L.pb254_verify_many_device.restype = C.c_int
+        L.pb254_verify_many_device.argtypes = [
+            C.c_void_p, C.c_int, C.POINTER(Config), C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_size_t,
+            C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_char)]
 
     def check(self, rc):
         if rc != 0:
@@ -398,6 +403,32 @@ class Context:
                                                     C.c_size_t(w.size), _p(inputs), _p(timestamps),
                                                     C.c_size_t(inputs.shape[0])))
         return True
+
+    def verify_many(self, kind, proofs, batches, config: Config | None = None):
+        """pb254_verify_many_device: :meth:`verify` on every proof, with one launch per stage for every 64 proofs.
+        `batches` is one (inputs, timestamps) per proof, of any sizes. Returns one entry per proof: None if accepted,
+        else (code, message), what :meth:`Library.verify` reports for that proof alone. Raises Pb254Error for bad
+        arguments and for a CUDA or out-of-memory error, which fails the whole call."""
+        if len(proofs) != len(batches):
+            raise Pb254Error(6, "one (inputs, timestamps) batch per proof")
+        args = [self.L._verify_args(kind, w, inp, ts) for w, (inp, ts) in zip(proofs, batches)]
+        n = len(args)
+        iw = self.L.input_words(kind)
+        inputs = np.concatenate([a[1] for a in args]) if n else np.empty((0, iw), dtype=np.uint64)
+        timestamps = np.concatenate([a[2] for a in args]) if n else np.empty(0, dtype=np.uint64)
+        starts = np.zeros(n + 1, dtype=np.uint64)
+        starts[1:] = np.cumsum([a[1].shape[0] for a in args])
+        words = (C.c_void_p * max(n, 1))(*[a[0].ctypes.data for a in args])
+        sizes = (C.c_size_t * max(n, 1))(*[a[0].size for a in args])
+        codes = (C.c_int * max(n, 1))(*([-1] * max(n, 1)))
+        msgs = C.create_string_buffer(max(n, 1) * MESSAGE_BYTES)
+        rc = self.L.lib.pb254_verify_many_device(self._h, kind, C.byref(config) if config is not None else None, words,
+                                                 sizes, n, _p(inputs), _p(timestamps), _p(starts), codes, msgs)
+        if rc in (4, 5) or any(codes[b] == -1 for b in range(n)):
+            self.L.check(rc)
+        return [None if codes[b] == 0 else
+                (codes[b], msgs.raw[b * MESSAGE_BYTES:(b + 1) * MESSAGE_BYTES].split(b"\0", 1)[0].decode())
+                for b in range(n)]
 
     def prove_sharded(self, kind, inputs, timestamps, rank: int, world: int, all_to_all, all_gather,
                       min_rows=1 << 16, config: Config | None = None):

@@ -16,6 +16,7 @@ pub const PB254_E_BAD_ARG: c_int = 6;
 pub const PB254_E_VERIFY: c_int = 7;
 pub const PB254_E_NOT_ON_CURVE: c_int = 8;
 pub const PB254_MAX_FRI_LAYERS: usize = 16;
+pub const PB254_VERIFY_MESSAGE_BYTES: usize = 256;
 
 /// `StarkConfig` (starky config.rs); `standard_fast_config()` = {1, 4, 2, 84, 16, 4, 5}.
 #[repr(C)]
@@ -139,6 +140,10 @@ extern "C" {
                         inputs: *const u64, timestamps: *const u64, n_inputs: usize) -> c_int;
     pub fn pb254_verify_device(ctx: *mut pb254_ctx, kind: c_int, cfg: *const pb254_config, proof_words: *const u64,
                                n_words: usize, inputs: *const u64, timestamps: *const u64, n_inputs: usize) -> c_int;
+    pub fn pb254_verify_many_device(ctx: *mut pb254_ctx, kind: c_int, cfg: *const pb254_config,
+                                    proof_words: *const *const u64, n_words: *const usize, n_proofs: usize,
+                                    inputs: *const u64, timestamps: *const u64, input_starts: *const u64,
+                                    codes_out: *mut c_int, messages_out: *mut c_char) -> c_int;
     pub fn pb254_proof_parse(proof_words: *const u64, n_words: usize, out: *mut pb254_proof_layout) -> c_int;
     pub fn pb254_proof_results_words(proof: *const pb254_proof) -> usize;
     pub fn pb254_proof_results_data(proof: *const pb254_proof) -> *const u64;

@@ -315,6 +315,44 @@ impl Context {
                                      blob.len(), words.as_ptr(), timestamps.as_ptr(), timestamps.len())
         })
     }
+
+    /// `verify` on every proof of one kind under one config (`pb254_verify_many_device`, one launch per stage for
+    /// every 64 proofs): `batches[b]` = (`pack_*` rows, timestamps) of `proofs[b]`, of any sizes. The outer error is a
+    /// bad argument or a CUDA / out-of-memory failure of the whole call; entry b is what `verify` returns for proof b.
+    pub fn verify_many(&self, kind: i32, config: Option<&StarkConfig>, proofs: &[&[u64]], batches: &[(&[u64], &[u64])])
+                       -> Result<Vec<Result<()>>> {
+        if proofs.len() != batches.len() {
+            return Err(anyhow!("pb254 error {}: one batch per proof", sys::PB254_E_BAD_ARG));
+        }
+        let cfg = config.map(config_of).transpose()?;
+        let n = proofs.len();
+        let ptrs: Vec<*const u64> = proofs.iter().map(|p| p.as_ptr()).collect();
+        let sizes: Vec<usize> = proofs.iter().map(|p| p.len()).collect();
+        let words: Vec<u64> = batches.iter().flat_map(|b| b.0.iter().copied()).collect();
+        let timestamps: Vec<u64> = batches.iter().flat_map(|b| b.1.iter().copied()).collect();
+        let mut starts = vec![0u64; n + 1];
+        for (b, batch) in batches.iter().enumerate() {
+            starts[b + 1] = starts[b] + batch.1.len() as u64;
+        }
+        let mut codes = vec![-1 as std::os::raw::c_int; n];
+        let mut msgs = vec![0 as std::os::raw::c_char; n * sys::PB254_VERIFY_MESSAGE_BYTES];
+        let rc = unsafe {
+            sys::pb254_verify_many_device(self.0, kind, cfg.as_ref().map_or(std::ptr::null(), |c| c as *const _),
+                                          ptrs.as_ptr(), sizes.as_ptr(), n, words.as_ptr(), timestamps.as_ptr(),
+                                          starts.as_ptr(), codes.as_mut_ptr(), msgs.as_mut_ptr())
+        };
+        if rc == sys::PB254_E_CUDA || rc == sys::PB254_E_OOM || codes.iter().any(|&c| c == -1) {
+            check(rc)?;
+        }
+        Ok(codes.iter().enumerate().map(|(b, &code)| {
+            if code == sys::PB254_OK {
+                return Ok(());
+            }
+            let slot = &msgs[b * sys::PB254_VERIFY_MESSAGE_BYTES..(b + 1) * sys::PB254_VERIFY_MESSAGE_BYTES];
+            let msg = unsafe { std::ffi::CStr::from_ptr(slot.as_ptr()) }.to_string_lossy().into_owned();
+            Err(anyhow!("pb254 error {code}: {msg}"))
+        }).collect())
+    }
 }
 impl Drop for Context {
     fn drop(&mut self) {
